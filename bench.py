@@ -41,7 +41,33 @@ def parse_args():
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--prompt", type=int, default=32, help="prompt tokens fed before the timed region (reference bench.rs:24)")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary measurements (prefill GEMM, batch-32)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (logits, next token ids) as DIR/<name>.npy, "
+                    "so that two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample of matvecs, not whole decode steps")
+    return args
+
+
+DUMP_LIMIT = 64_000_000  # bytes on disk, all files of one dump together
+
+
+def write_outputs(out_dir: str, arrays: dict, limit: int = DUMP_LIMIT):
+    """Each array goes to out_dir/<name>.npy as float32 (float64 for 64-bit inputs such as token ids, which it holds exactly).
+    An array larger than its share of `limit` bytes is replaced by a fixed sample of its flattened elements (seeded, so the
+    same elements for the same shape on every run and every build) and the sample's flat indices go to <name>_index.npy."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = limit // len(arrays) - 256  # room for the .npy headers of an array and its index
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64 if a.dtype.itemsize == 8 else np.float32)
+        if a.nbytes > share:
+            rng = np.random.Generator(np.random.PCG64(a.size))
+            idx = np.sort(rng.choice(a.size, share // (a.itemsize + 8), replace=False))
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peaks():
@@ -231,6 +257,10 @@ def run_b200(args):
     barrier()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    outputs = None
+    if args.dump_outputs and rank == 0:  # taken now: the end-to-end loop below decodes further tokens into the same buffers
+        logits = dec.logits_local if emu > 1 and world == 1 else dec.full_logits()
+        outputs = {"logits": logits.cpu().numpy(), "next_ids": dec.ids.cpu().numpy()}
 
     # ---- end to end through the step API with host buffers ----
     pin_in = torch.zeros(M, dtype=torch.int64).pin_memory()
@@ -347,6 +377,8 @@ def run_b200(args):
             out["cpu_baseline"] = {"value": cpu_v, "unit": "tokens/s", "cores": cores, "kind": "port", "sample": sample}
         if extra:
             out["extra"] = extra
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(out), flush=True)
     watchdog.cancel()
     if world > 1:
