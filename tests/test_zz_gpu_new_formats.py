@@ -7,10 +7,9 @@ import pytest
 
 import test_gpu_gemm as tg
 import test_gpu_quant as tq
+from qcases import NEW
 
 pytestmark = [pytest.mark.gpu]
-
-NEW = ["Q5_K", "Q4_1", "Q5_1", "Q2_K", "Q3_K", "IQ4_XS", "TQ2_0", "TQ1_0", "IQ2_XXS", "IQ2_XS", "IQ3_XXS", "IQ2_S", "IQ3_S", "IQ1_S", "IQ1_M"]
 
 
 @pytest.mark.parametrize("name", NEW)
@@ -42,7 +41,7 @@ def test_matvec_small_batch(client, fmt, M):
 
 
 @pytest.mark.parametrize("fmt", NEW)
-@pytest.mark.parametrize("NKM", [(128, 256, 32), (200, 768, 100), (384, 4096, 256)])
+@pytest.mark.parametrize("NKM", [(128, 256, 32), (200, 768, 100), (384, 4096, 256), (256, 14336, 64)])
 def test_gemm_vs_oracle(client, fmt, NKM):
     tg.test_gemm_vs_oracle(client, fmt, NKM)
 
