@@ -269,6 +269,9 @@ __global__ void __launch_bounds__(256) swiglu_quant_kernel(const float* __restri
 // token; rope: [max_ctx][hd/2][2] (cos, sin).  One CTA of ATT_NT threads per (head, m); dynamic smem = max_ctx f32.
 // ------------------------------------------------------------------------------------------------
 constexpr int ATT_NT = 512;  // threads per (head, m): 128 positions per score sweep, so a short context is one round trip
+constexpr int ATTN_SINGLE_MAX_CTX = 160 * 1024 / 4;   // the single-CTA kernel's score buffer: 160 KB of dynamic shared memory
+constexpr int ATTN_SPLIT_MIN = 256;   // split-context kernels: fewest positions per split (short contexts use fewer CTAs)
+constexpr int ATTN_SPLIT_CAP = 128;   // ... and most splits per (kv head, sequence); longer contexts get longer splits
 // PAGED (reference src/engine/batch_decode.rs:77-147, forward_with_paged_kv_cache): cache_k / cache_v are block POOLS
 // [num_blocks][block_size][nkv][hd]; position j of sequence m lives in block block_table[m][j / block_size] at offset
 // j % block_size; the new token goes to slot_mapping[m] (= block * block_size + offset; derived from the block table when
@@ -466,6 +469,349 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
         }
         gt.done();
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Split-context decode attention: the same definition as attn_decode_kernel for any max_ctx (the single-CTA kernel keeps
+// every score of a (head, m) in shared memory, so it stops at ATTN_SINGLE_MAX_CTX positions).  Three PDL-chained kernels
+// over a caller-provided workspace:
+//   A  attn_split_scores_kernel  grid (nkv, M, S_max): split s of the positions [0, p] of sequence m; ONE CTA serves all
+//      G = nh / nkv query heads of its kv head (every K row is read once and dotted with G rotated queries).  Writes the
+//      f32 scores [M][nh][max_ctx] and each split's maximum [M][nh][S_max].  The CTA owning position p appends the new row.
+//   B  attn_split_pv_kernel      same grid: global maximum = max of the split maxima, p_j = det_exp(s_j - max), f64
+//      partials sum_j p_j and sum_j p_j v_j of the split -> [M][nh][S_max] and [M][nh][S_max][hd].
+//   C  attn_split_combine_kernel grid (nh, M): partials summed in split order, one division, attn_out / xq records.
+// Scores are bit-identical to the single-CTA kernel's (same f64 operation order of each dot product, same f32 rounding and
+// scale); only the order of the f64 sums of pass 2 differs (DESIGN section 2 contract 3: invisible up to 1e-16).  Split
+// boundaries are a function of p only (attn_split_range), so results are deterministic; the launch shape depends only on
+// max_ctx (graph-capturable).  No reader ever reads row p from the cache (the new k / v come from qkv), so the append in
+// kernel A cannot race with the other CTAs.
+// ------------------------------------------------------------------------------------------------
+constexpr int ATT_SPLIT_NT = 256;       // threads per split CTA (kernels A and B)
+constexpr int ATT_SPLIT_GC = 8;         // query heads per pass over a split's rows (G > 8 makes ceil(G / 8) passes)
+constexpr int ATT_SPLIT_TILE = 64;      // kernel B: positions whose probabilities are staged in shared memory at a time
+
+__host__ __device__ __forceinline__ int attn_split_max(int max_ctx) {
+    const int s = (int)(((int64_t)max_ctx + ATTN_SPLIT_MIN - 1) / ATTN_SPLIT_MIN);
+    return s < ATTN_SPLIT_CAP ? s : ATTN_SPLIT_CAP;
+}
+// split s of the positions [0, p]: S_eff = min(S_max, ceil((p + 1) / ATTN_SPLIT_MIN)) balanced ranges [j0, j1); s >= S_eff -> empty
+__device__ __forceinline__ void attn_split_range(int p, int s_max, int s, int& j0, int& j1, int& s_eff) {
+    const int64_t n = (int64_t)p + 1;
+    const int64_t want = (n + ATTN_SPLIT_MIN - 1) / ATTN_SPLIT_MIN;
+    s_eff = (int)(want < s_max ? want : s_max);
+    if (s >= s_eff) { j0 = j1 = 0; return; }
+    j0 = (int)((int64_t)s * n / s_eff);
+    j1 = (int)((int64_t)(s + 1) * n / s_eff);
+}
+
+struct AttnSplitWs {
+    float* scores;    // [M][nh][max_ctx]
+    float* smax;      // [M][nh][S_max]
+    double* psum;     // [M][nh][S_max]
+    double* pv;       // [M][nh][S_max][hd]
+};
+
+// the position checks of attn_decode_kernel: the same clamped position ahead of the wait, and the same verdict in all three kernels
+template <bool PAGED>
+__device__ __forceinline__ int attn_checked_pos(const int* pos, int m, int max_ctx, const PagedKv& pg, bool& bad_pos) {
+    const int p_raw = pos[m];
+    bad_pos = p_raw < 0 || p_raw >= max_ctx;
+    if constexpr (PAGED) {
+        if (pg.slot_mapping && pg.slot_mapping[m] < 0) bad_pos = true;
+    }
+    return bad_pos ? 0 : p_raw;
+}
+
+template <int HD, bool PAGED>
+__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, float* __restrict__ cache_k,
+                                                                       float* __restrict__ cache_v, const float* __restrict__ rope, int nh, int nkv, int max_ctx,
+                                                                       const PagedKv pg, const AttnSplitWs ws) {
+    pdl_launch_dependents();
+    const int kvh = blockIdx.x, m = blockIdx.y, s = blockIdx.z, t = threadIdx.x, warp = t >> 5, lane = t & 31;
+    const int G = nh / nkv, s_max = gridDim.z;
+    constexpr int QE = HD / 4;          // elements per thread: 4 threads per position, a quarter of the head each
+    constexpr int QP = QE + 2;          // padded quarter (doubles): the 4 quarters of a query fall in different banks
+    constexpr int NW = ATT_SPLIT_NT / 32;
+    bool bad_pos;
+    const int p = attn_checked_pos<PAGED>(pos, m, max_ctx, pg, bad_pos);
+    int j0, j1, s_eff;
+    attn_split_range(p, s_max, s, j0, j1, s_eff);
+    const int row = (nh + 2 * nkv) * HD;
+    const float* ksrc = qkv + (size_t)m * row + (size_t)(nh + kvh) * HD;
+    const float* vsrc = qkv + (size_t)m * row + (size_t)(nh + nkv + kvh) * HD;
+    const size_t pstride = (size_t)nkv * HD;
+    const int* bt = PAGED ? pg.block_table + (size_t)m * pg.max_blocks : nullptr;
+    auto row_of = [&](int j) -> size_t {
+        if constexpr (PAGED) return ((size_t)bt[j / pg.block_size] * pg.block_size + (size_t)(j % pg.block_size)) * pstride + (size_t)kvh * HD;
+        else return ((size_t)m * max_ctx + (size_t)j) * pstride + (size_t)kvh * HD;
+    };
+    const float* rt = rope + (size_t)p * HD;
+    __shared__ __align__(16) double sq[ATT_SPLIT_GC][4][QP];
+    __shared__ __align__(16) float sk[HD];
+    __shared__ float s_red[NW][ATT_SPLIT_GC];
+    pdl_wait();
+    if (bad_pos) {
+        if (t == 0 && s == 0 && kvh == 0) atomicOr(&g_decode_error, B200Q_DECODE_ERR_POSITION);
+        return;
+    }
+    if (s >= s_eff) return;
+    const bool owns_p = j1 == p + 1;
+    if (t < HD / 2) {   // the new key, rotated exactly as attn_decode_kernel does (it is scored from here, never from the cache)
+        const float c = rt[2 * t], sn = rt[2 * t + 1];
+        const float k0 = ksrc[2 * t], k1 = ksrc[2 * t + 1];
+        const float r0 = __fsub_rn(__fmul_rn(k0, c), __fmul_rn(k1, sn)), r1 = __fadd_rn(__fmul_rn(k0, sn), __fmul_rn(k1, c));
+        sk[2 * t] = r0; sk[2 * t + 1] = r1;
+        if (owns_p) {
+            size_t wrow = row_of(p);
+            if constexpr (PAGED) {
+                if (pg.slot_mapping) wrow = (size_t)pg.slot_mapping[m] * pstride + (size_t)kvh * HD;
+            }
+            cache_k[wrow + 2 * t] = r0; cache_k[wrow + 2 * t + 1] = r1;
+            cache_v[wrow + 2 * t] = vsrc[2 * t]; cache_v[wrow + 2 * t + 1] = vsrc[2 * t + 1];
+        }
+    }
+    const float scale = __fdiv_rn(1.0f, __fsqrt_rn((float)HD));
+    const int part = t & 3;
+    for (int g0 = 0; g0 < G; g0 += ATT_SPLIT_GC) {
+        const int gc = min(ATT_SPLIT_GC, G - g0);
+        __syncthreads();   // sk is written / the previous pass is done with sq and s_red
+        for (int i = t; i < gc * (HD / 2); i += ATT_SPLIT_NT) {
+            const int g = i / (HD / 2), e2 = 2 * (i % (HD / 2));
+            const float* qsrc = qkv + (size_t)m * row + (size_t)(kvh * G + g0 + g) * HD;
+            const float c = rt[e2], sn = rt[e2 + 1];
+            const float q0 = qsrc[e2], q1 = qsrc[e2 + 1];
+            sq[g][e2 / QE][e2 % QE] = (double)__fsub_rn(__fmul_rn(q0, c), __fmul_rn(q1, sn));
+            sq[g][e2 / QE][e2 % QE + 1] = (double)__fadd_rn(__fmul_rn(q0, sn), __fmul_rn(q1, c));
+        }
+        __syncthreads();
+        float lmax[ATT_SPLIT_GC];
+#pragma unroll
+        for (int g = 0; g < ATT_SPLIT_GC; g++) lmax[g] = -INFINITY;
+        float* sc_out = ws.scores + ((size_t)m * nh + (size_t)kvh * G + g0) * (size_t)max_ctx;
+        // 4 threads per position; a warp's 8 positions are processed together (the shuffles need the whole warp)
+        for (int jb = j0; jb < j1; jb += ATT_SPLIT_NT / 4) {
+            const int j = jb + (t >> 2);
+            const bool live = j < j1;
+            double kd[QE];
+            if (live) {
+                const float* kr = (j < p) ? cache_k + row_of(j) + part * QE : sk + part * QE;
+#pragma unroll
+                for (int e = 0; e < QE; e += 4) {
+                    const float4 kk = *reinterpret_cast<const float4*>(kr + e);
+                    kd[e] = (double)kk.x; kd[e + 1] = (double)kk.y; kd[e + 2] = (double)kk.z; kd[e + 3] = (double)kk.w;
+                }
+            } else {
+#pragma unroll
+                for (int e = 0; e < QE; e++) kd[e] = 0.0;
+            }
+#pragma unroll
+            for (int g = 0; g < ATT_SPLIT_GC; g++) {
+                if (g < gc) {
+                    // attn_decode_kernel's operation order: 4 fma chains over e mod 4, (d0+d1)+(d2+d3), then (P0+P1)+(P2+P3)
+                    const double* qq = sq[g][part];
+                    double d0 = 0.0, d1 = 0.0, d2 = 0.0, d3 = 0.0;
+#pragma unroll
+                    for (int e = 0; e < QE; e += 4) {
+                        d0 = fma(qq[e + 0], kd[e + 0], d0); d1 = fma(qq[e + 1], kd[e + 1], d1);
+                        d2 = fma(qq[e + 2], kd[e + 2], d2); d3 = fma(qq[e + 3], kd[e + 3], d3);
+                    }
+                    double d = (d0 + d1) + (d2 + d3);
+                    d += __shfl_xor_sync(0xffffffffu, d, 1);
+                    d += __shfl_xor_sync(0xffffffffu, d, 2);
+                    if (live) {
+                        const float sc = __fmul_rn((float)d, scale);
+                        if (part == (g & 3)) sc_out[(size_t)g * max_ctx + j] = sc;
+                        lmax[g] = fmaxf(lmax[g], sc);
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int g = 0; g < ATT_SPLIT_GC; g++) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) lmax[g] = fmaxf(lmax[g], __shfl_xor_sync(0xffffffffu, lmax[g], off));
+            if (lane == 0) s_red[warp][g] = lmax[g];
+        }
+        __syncthreads();
+        if (t < gc) {
+            float mx = s_red[0][t];
+#pragma unroll
+            for (int w = 1; w < NW; w++) mx = fmaxf(mx, s_red[w][t]);
+            ws.smax[((size_t)m * nh + (size_t)kvh * G + g0 + t) * s_max + s] = mx;
+        }
+    }
+}
+
+template <int HD, bool PAGED>
+__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_pv_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, const float* __restrict__ cache_v,
+                                                                   int nh, int nkv, int max_ctx, const PagedKv pg, const AttnSplitWs ws) {
+    pdl_launch_dependents();
+    const int kvh = blockIdx.x, m = blockIdx.y, s = blockIdx.z, t = threadIdx.x, warp = t >> 5, lane = t & 31;
+    const int G = nh / nkv, s_max = gridDim.z;
+    constexpr int EG = HD / 4;                 // element groups of 4 (one float4 of a V row)
+    constexpr int JG = ATT_SPLIT_NT / EG;      // position lanes: 8 for hd 128, 16 for hd 64 (adjacent lanes of a warp)
+    constexpr int NW = ATT_SPLIT_NT / 32;
+    const int jg = t % JG, eg = t / JG;
+    bool bad_pos;
+    const int p = attn_checked_pos<PAGED>(pos, m, max_ctx, pg, bad_pos);
+    int j0, j1, s_eff;
+    attn_split_range(p, s_max, s, j0, j1, s_eff);
+    const int row = (nh + 2 * nkv) * HD;
+    const float* vsrc = qkv + (size_t)m * row + (size_t)(nh + nkv + kvh) * HD;
+    const size_t pstride = (size_t)nkv * HD;
+    const int* bt = PAGED ? pg.block_table + (size_t)m * pg.max_blocks : nullptr;
+    auto row_of = [&](int j) -> size_t {
+        if constexpr (PAGED) return ((size_t)bt[j / pg.block_size] * pg.block_size + (size_t)(j % pg.block_size)) * pstride + (size_t)kvh * HD;
+        else return ((size_t)m * max_ctx + (size_t)j) * pstride + (size_t)kvh * HD;
+    };
+    __shared__ float sp[ATT_SPLIT_GC][ATT_SPLIT_TILE];
+    __shared__ float gmax[ATT_SPLIT_GC];
+    __shared__ __align__(16) float sv[HD];
+    __shared__ double s_red[2][NW];
+    pdl_wait();
+    if (bad_pos || s >= s_eff) return;
+    for (int i = t; i < HD; i += ATT_SPLIT_NT) sv[i] = vsrc[i];
+    for (int g0 = 0; g0 < G; g0 += ATT_SPLIT_GC) {
+        const int gc = min(ATT_SPLIT_GC, G - g0);
+        const size_t hrow = (size_t)m * nh + (size_t)kvh * G + g0;   // first (m, head) row of this pass
+        __syncthreads();
+        if (t < gc) {
+            const float* sm = ws.smax + (hrow + t) * s_max;
+            float mx = sm[0];
+            for (int i = 1; i < s_eff; i++) mx = fmaxf(mx, sm[i]);
+            gmax[t] = mx;
+        }
+        double o[ATT_SPLIT_GC][4];
+#pragma unroll
+        for (int g = 0; g < ATT_SPLIT_GC; g++) o[g][0] = o[g][1] = o[g][2] = o[g][3] = 0.0;
+        double ls0 = 0.0, ls1 = 0.0;   // sum of p of heads t / 64 and 4 + t / 64
+        for (int jt = j0; jt < j1; jt += ATT_SPLIT_TILE) {
+            __syncthreads();   // gmax ready / the previous tile's probabilities are consumed
+            {
+                const int jj = t % ATT_SPLIT_TILE, g = t / ATT_SPLIT_TILE, j = jt + jj;
+                static_assert(ATT_SPLIT_NT == 4 * ATT_SPLIT_TILE && ATT_SPLIT_GC == 8, "two probabilities per thread");
+                float pa = 0.0f, pb = 0.0f;
+                if (j < j1) {
+                    if (g < gc) pa = det_expf(__fsub_rn(ws.scores[(hrow + g) * max_ctx + j], gmax[g]));
+                    if (g + 4 < gc) pb = det_expf(__fsub_rn(ws.scores[(hrow + g + 4) * max_ctx + j], gmax[g + 4]));
+                }
+                sp[g][jj] = pa; sp[g + 4][jj] = pb;
+                ls0 += (double)pa; ls1 += (double)pb;
+            }
+            __syncthreads();
+            const int jn = min(ATT_SPLIT_TILE, j1 - jt);
+            for (int jj = jg; jj < jn; jj += JG) {
+                const int j = jt + jj;
+                const float4 vv = (j < p) ? *reinterpret_cast<const float4*>(cache_v + row_of(j) + 4 * eg) : *reinterpret_cast<const float4*>(sv + 4 * eg);
+#pragma unroll
+                for (int g = 0; g < ATT_SPLIT_GC; g++) {
+                    const double pj = (double)sp[g][jj];
+                    o[g][0] = fma(pj, (double)vv.x, o[g][0]); o[g][1] = fma(pj, (double)vv.y, o[g][1]);
+                    o[g][2] = fma(pj, (double)vv.z, o[g][2]); o[g][3] = fma(pj, (double)vv.w, o[g][3]);
+                }
+            }
+        }
+        // the JG position lanes of an element group are adjacent lanes of one warp
+#pragma unroll
+        for (int g = 0; g < ATT_SPLIT_GC; g++)
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+                for (int off = 1; off < JG; off <<= 1) o[g][i] += __shfl_xor_sync(0xffffffffu, o[g][i], off);
+        if (jg == 0) {
+#pragma unroll
+            for (int g = 0; g < ATT_SPLIT_GC; g++)
+                if (g < gc) {
+                    double* dst = ws.pv + ((hrow + g) * s_max + s) * HD + 4 * eg;
+                    dst[0] = o[g][0]; dst[1] = o[g][1]; dst[2] = o[g][2]; dst[3] = o[g][3];
+                }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            ls0 += __shfl_xor_sync(0xffffffffu, ls0, off);
+            ls1 += __shfl_xor_sync(0xffffffffu, ls1, off);
+        }
+        if (lane == 0) { s_red[0][warp] = ls0; s_red[1][warp] = ls1; }
+        __syncthreads();
+        if (t < gc) {   // warps 2 h and 2 h + 1 hold head h (h < 4) in s_red[0] and head h + 4 in s_red[1]
+            const int hb = t & 3, k = t >> 2;
+            ws.psum[(hrow + t) * s_max + s] = s_red[k][2 * hb] + s_red[k][2 * hb + 1];
+        }
+    }
+}
+
+template <int HD, bool PAGED>
+__global__ void __launch_bounds__(HD) attn_split_combine_kernel(const int* __restrict__ pos, int nh, int max_ctx, int s_max, int M, const PagedKv pg,
+                                                               const AttnSplitWs ws, uint8_t* __restrict__ xq, float* __restrict__ attn_out) {
+    pdl_launch_dependents();
+    const int head = blockIdx.x, m = blockIdx.y, t = threadIdx.x, lane = t & 31;
+    bool bad_pos;
+    const int p = attn_checked_pos<PAGED>(pos, m, max_ctx, pg, bad_pos);
+    int j0, j1, s_eff;
+    attn_split_range(p, s_max, 0, j0, j1, s_eff);
+    pdl_wait();
+    if (bad_pos) return;
+    const size_t hrow = (size_t)m * nh + head;
+    double o = 0.0, dsum = 0.0;
+    const double* pv = ws.pv + hrow * s_max * HD + t;
+    const double* ps = ws.psum + hrow * s_max;
+#pragma unroll 8
+    for (int i = 0; i < s_eff; i++) {   // split order
+        o += pv[(size_t)i * HD];
+        dsum += ps[i];
+    }
+    const float outv = __fdiv_rn((float)o, (float)dsum);
+    if (attn_out) attn_out[(size_t)m * nh * HD + (size_t)head * HD + t] = outv;
+    if (!xq) return;
+    // the o_proj activation records, quantised as attn_decode_kernel does (32-blocks never straddle heads)
+    const int kglob = head * HD + t;
+    const int kc = kglob / CHUNK_K, tin = kglob % CHUNK_K;
+    uint8_t* rec = xq + ((size_t)kc * M + m) * ACT_REC_BYTES;
+    float amax = fabsf(outv);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, off));
+    const float d = __fdiv_rn(amax, 127.0f);
+    const float id = (d != 0.0f) ? __fdiv_rn(1.0f, d) : 0.0f;
+    const int q = (int)roundf(__fmul_rn(outv, id));
+    int sm = q;
+#pragma unroll
+    for (int off = 8; off > 0; off >>= 1) sm += __shfl_xor_sync(0xffffffffu, sm, off);
+    const int s_hi = __shfl_sync(0xffffffffu, sm, 16);
+    rec[tin] = (uint8_t)(int8_t)q;
+    if (lane == 0) {
+        reinterpret_cast<float*>(rec + 256)[tin >> 5] = d;
+        reinterpret_cast<uint32_t*>(rec + 288)[tin >> 5] = ((uint32_t)sm & 0xFFFFu) | ((uint32_t)s_hi << 16);
+    }
+}
+
+// workspace regions, each 256-byte aligned; returns the total (0 for arguments no split kernel accepts)
+static size_t attn_split_layout(int64_t nh, int64_t hd, int64_t max_ctx, int64_t M, uint8_t* base, AttnSplitWs* ws) {
+    if (nh <= 0 || max_ctx <= 0 || M <= 0 || (hd != 64 && hd != 128)) return 0;
+    const size_t smax = (size_t)attn_split_max((int)max_ctx);
+    const size_t rows = (size_t)M * (size_t)nh;
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_sc = al(rows * (size_t)max_ctx * 4), b_mx = al(rows * smax * 4), b_ps = al(rows * smax * 8), b_pv = al(rows * smax * (size_t)hd * 8);
+    if (ws) {
+        ws->scores = reinterpret_cast<float*>(base);
+        ws->smax = reinterpret_cast<float*>(base + b_sc);
+        ws->psum = reinterpret_cast<double*>(base + b_sc + b_mx);
+        ws->pv = reinterpret_cast<double*>(base + b_sc + b_mx + b_ps);
+    }
+    return b_sc + b_mx + b_ps + b_pv;
+}
+
+template <int HD, bool PAGED>
+static cudaError_t launch_attn_split(const float* qkv, const int* pos, float* ck, float* cv, const float* rope, int nh, int nkv, int max_ctx, int M,
+                                     uint8_t* xq, float* attn_out, const PagedKv& pg, const AttnSplitWs& ws, cudaStream_t st) {
+    const int s_max = attn_split_max(max_ctx);
+    const dim3 grid((unsigned)nkv, (unsigned)M, (unsigned)s_max);
+    cudaError_t e = launch_pdl(attn_split_scores_kernel<HD, PAGED>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, ck, cv, rope, nh, nkv, max_ctx, pg, ws);
+    if (e == cudaSuccess)
+        e = launch_pdl(attn_split_pv_kernel<HD, PAGED>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, (const float*)cv, nh, nkv, max_ctx, pg, ws);
+    if (e == cudaSuccess)
+        e = launch_pdl(attn_split_combine_kernel<HD, PAGED>, dim3((unsigned)nh, (unsigned)M), dim3(HD), 0, st, pos, nh, max_ctx, s_max, M, pg, ws, xq, attn_out);
+    return e;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -673,7 +1019,7 @@ int32_t b200q_attn_decode(const float* qkv, const int32_t* pos, float* cache_k, 
     if (!qkv || !pos || !cache_k || !cache_v || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 || max_ctx <= 0)
         return B200Q_ERR_INVALID_ARG;
     if (((int64_t)n_heads * head_dim) % CHUNK_K) return B200Q_ERR_INVALID_ARG;
-    if ((size_t)max_ctx * 4 > 160 * 1024) return B200Q_ERR_UNSUPPORTED;
+    if (max_ctx > ATTN_SINGLE_MAX_CTX) return B200Q_ERR_UNSUPPORTED;
     cudaError_t e;
     dim3 grid((unsigned)n_heads, (unsigned)M);
     size_t smem = (size_t)max_ctx * sizeof(float);
@@ -705,7 +1051,7 @@ int32_t b200q_attn_decode_paged(const float* qkv, const int32_t* pos, float* k_p
         return B200Q_ERR_INVALID_ARG;
     if (((int64_t)n_heads * head_dim) % CHUNK_K) return B200Q_ERR_INVALID_ARG;
     const int64_t max_ctx = (int64_t)block_size * max_blocks;
-    if ((size_t)max_ctx * 4 > 160 * 1024) return B200Q_ERR_UNSUPPORTED;
+    if (max_ctx > ATTN_SINGLE_MAX_CTX) return B200Q_ERR_UNSUPPORTED;
     cudaError_t e;
     dim3 grid((unsigned)n_heads, (unsigned)M);
     size_t smem = (size_t)max_ctx * sizeof(float);
@@ -722,6 +1068,59 @@ int32_t b200q_attn_decode_paged(const float* qkv, const int32_t* pos, float* k_p
         return B200Q_ERR_UNSUPPORTED;
     }
     return e == cudaSuccess ? B200Q_OK : B200Q_ERR_CUDA;
+}
+
+int32_t b200q_attn_decode_max_ctx(void) { return ATTN_SINGLE_MAX_CTX; }
+
+size_t b200q_attn_split_workspace_bytes(int32_t n_heads, int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M) {
+    if (n_kv_heads <= 0 || n_heads % n_kv_heads) return 0;
+    return attn_split_layout(n_heads, head_dim, max_ctx, M, nullptr, nullptr);
+}
+
+static int32_t attn_split_dispatch(const float* qkv, const int32_t* pos, float* ck, float* cv, const float* rope, int32_t nh, int32_t nkv, int32_t hd,
+                                   int64_t max_ctx, int64_t M, void* xq, float* attn_out, const PagedKv& pg, void* workspace, size_t workspace_bytes,
+                                   void* stream, const char* who) {
+    if (hd != 64 && hd != 128) return set_error(B200Q_ERR_UNSUPPORTED, "%s: head_dim %d (64 or 128)", who, (int)hd);
+    if (max_ctx > INT32_MAX || M > 65535) return set_error(B200Q_ERR_INVALID_ARG, "%s: max_ctx %lld / M %lld out of range", who, (long long)max_ctx, (long long)M);
+    AttnSplitWs ws;
+    const size_t need = attn_split_layout(nh, hd, max_ctx, M, (uint8_t*)workspace, &ws);
+    if (!workspace || workspace_bytes < need)
+        return set_error(B200Q_ERR_WORKSPACE, "%s: workspace of %zu bytes, %zu needed (b200q_attn_split_workspace_bytes)", who, workspace_bytes, need);
+    cudaError_t e;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const bool paged = pg.block_table != nullptr;
+    if (hd == 128)
+        e = paged ? launch_attn_split<128, true>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st)
+                  : launch_attn_split<128, false>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st);
+    else
+        e = paged ? launch_attn_split<64, true>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st)
+                  : launch_attn_split<64, false>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st);
+    return e == cudaSuccess ? B200Q_OK : set_error(B200Q_ERR_CUDA, "%s launch: %s", who, cudaGetErrorString(e));
+}
+
+/* Split-context form of b200q_attn_decode for any max_ctx >= 1 (same arguments, same results up to the order of the f64 sums). */
+int32_t b200q_attn_decode_split(const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table, int32_t n_heads,
+                                int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+    if (!qkv || !pos || !cache_k || !cache_v || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 || max_ctx <= 0)
+        return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_split: bad arguments");
+    if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_split: n_heads * head_dim not a multiple of %d", CHUNK_K);
+    const PagedKv none{nullptr, nullptr, 0, 0};
+    return attn_split_dispatch(qkv, pos, cache_k, cache_v, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, none, workspace,
+                               workspace_bytes, stream, "attn_decode_split");
+}
+
+/* Split-context form of b200q_attn_decode_paged; max_ctx = block_size * max_blocks sizes the workspace. */
+int32_t b200q_attn_decode_paged_split(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
+                                      int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
+                                      int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!qkv || !pos || !k_pool || !v_pool || !block_table || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 ||
+        block_size <= 0 || max_blocks <= 0)
+        return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged_split: bad arguments");
+    if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged_split: n_heads * head_dim not a multiple of %d", CHUNK_K);
+    const PagedKv pg{block_table, slot_mapping, block_size, max_blocks};
+    return attn_split_dispatch(qkv, pos, k_pool, v_pool, rope_table, n_heads, n_kv_heads, head_dim, (int64_t)block_size * max_blocks, M, xq, attn_out, pg,
+                               workspace, workspace_bytes, stream, "attn_decode_paged_split");
 }
 
 /* Reads and clears the sticky device error word of the CURRENT device (synchronises the device: call it outside

@@ -19,7 +19,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, field
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 import torch
@@ -39,6 +39,9 @@ class ModelConfig:
     vocab: int
     rope_theta: float = 10000.0
     eps: float = 1e-5
+    # Llama 3.1 / 3.2 ("llama3" rope scaling): per-frequency divisors of the RoPE frequencies, head_dim / 2 values
+    # (llama.cpp stores them as the rope_freqs.weight tensor); None = unscaled
+    rope_freq_factors: Optional[Tuple[float, ...]] = None
 
 
 PRESETS: Dict[str, ModelConfig] = {
@@ -52,11 +55,15 @@ PRESETS: Dict[str, ModelConfig] = {
 }
 
 
-def rope_table(max_ctx: int, head_dim: int, theta: float) -> np.ndarray:
-    """[max_ctx, hd/2, 2] f32 (cos, sin) of pos * theta^(-2i/hd), computed in f64 and rounded once.  The same
-    formula is restated in oracle/model.py; a table (instead of device powf/sincos) keeps RoPE bit-reproducible."""
+def rope_table(max_ctx: int, head_dim: int, theta: float, factors=None) -> np.ndarray:
+    """[max_ctx, hd/2, 2] f32 (cos, sin) of pos * theta^(-2i/hd) / factors[i], computed in f64 and rounded once.  The same
+    formula is restated in oracle/model.py (unscaled) and tests/rope_ref.py (with factors); a table (instead of device
+    powf/sincos) keeps RoPE bit-reproducible.
+    factors: the Llama 3.1 / 3.2 frequency divisors (ggml divides theta by them); None leaves the frequencies unscaled."""
     i = np.arange(head_dim // 2, dtype=np.float64)
     freq = np.power(float(theta), -2.0 * i / head_dim)
+    if factors is not None:
+        freq = freq / np.asarray(factors, dtype=np.float64).reshape(head_dim // 2)
     ang = np.arange(max_ctx, dtype=np.float64)[:, None] * freq[None, :]
     return np.stack([np.cos(ang), np.sin(ang)], axis=-1).astype(np.float32)
 
@@ -259,7 +266,19 @@ class Decoder:
                 lay["cv"] = torch.zeros((M, max_ctx, self.nkv, hd), dtype=torch.float32, device=dev)
             self.layers.append(lay)
         self.final_norm = torch.from_numpy(host.final_norm if host else np.ones(H, np.float32)).to(dev)
-        self.rope = torch.from_numpy(rope_table(max_ctx, hd, cfg.rope_theta)).to(dev)
+        self.rope = torch.from_numpy(rope_table(max_ctx, hd, cfg.rope_theta, cfg.rope_freq_factors)).to(dev)
+        # decode attention: the single-CTA kernel holds every score of a (head, sequence) in shared memory; past its limit the
+        # split-context kernels run over one workspace shared by all layers (they run in sequence on one stream)
+        self.attn_split = max_ctx > int(ops.lib().b200q_attn_decode_max_ctx())
+        self.attn_ws = None
+        if self.attn_split:
+            if dstep:
+                raise ValueError(f"max_ctx={max_ctx} exceeds the op-list kernel's attention limit "
+                                 f"({int(ops.lib().b200q_attn_decode_max_ctx())}): unset B200Q_DSTEP")
+            nbytes = int(ops.lib().b200q_attn_split_workspace_bytes(self.nh, self.nkv, hd, max_ctx, M))
+            if nbytes == 0:
+                raise ValueError(f"split-context attention does not support head_dim {hd}")
+            self.attn_ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
         self.head = self._fused(-1, [("lm_head", host.lm_head.fmt if host else head_format(scheme), cfg.vocab, v0, v1 - v0)], H, host)
         if host is not None:
             self.embed = torch.from_numpy(host.embed).to(dev)
@@ -534,6 +553,18 @@ class Decoder:
         L, cfg, M = ops.lib(), self.cfg, self.M
         P = lambda t: C.c_void_p(t.data_ptr())
         xq, ao = (None, P(self.xq_attn)) if self.wide else (P(self.xq_attn), None)
+        if self.attn_split:
+            ws, wsb = P(self.attn_ws), C.c_size_t(self.attn_ws.numel())
+            if self.paged:
+                ops._check(L.b200q_attn_decode_paged_split(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.block_table),
+                                                           P(self.slot_mapping) if self.slot_mapping is not None else None,
+                                                           C.c_int32(self.block_size), C.c_int32(self.max_blocks), P(self.rope), C.c_int32(self.nh),
+                                                           C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int64(M), xq, ao, ws, wsb, st))
+            else:
+                ops._check(L.b200q_attn_decode_split(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.rope), C.c_int32(self.nh),
+                                                     C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M), xq, ao,
+                                                     ws, wsb, st))
+            return
         if self.paged:
             ops._check(L.b200q_attn_decode_paged(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.block_table),
                                                  P(self.slot_mapping) if self.slot_mapping is not None else None, C.c_int32(self.block_size),
@@ -701,7 +732,7 @@ class Decoder:
         sw = 0 if self.fused_swiglu else 1
         n = 1 + glue + len(self.head) + 1  # embed, (final norm), head, argmax
         for lay in self.layers:
-            n += 2 * glue + len(lay["qkv"]) + 1 + len(lay["o"]) + len(lay["gu"]) + sw + len(lay["down"])
+            n += 2 * glue + len(lay["qkv"]) + (3 if self.attn_split else 1) + len(lay["o"]) + len(lay["gu"]) + sw + len(lay["down"])
         return n
 
     def capture(self):

@@ -276,6 +276,20 @@ def config_from_gguf_metadata(g: Gguf):
 SUPPORTED_DECODER_ARCHS = frozenset({"llama", "mistral"})
 
 
+def rope_freq_factors(g: Gguf, head_dim: int) -> Tuple[float, ...]:
+    """the per-frequency RoPE divisors llama.cpp's converter writes as rope_freqs.weight for models trained with
+    rope_scaling.rope_type "llama3" (Llama 3.1 / 3.2): F32, shape (head_dim / 2,), finite and positive -- anything else raises"""
+    ti = g.tensor_info("rope_freqs.weight")
+    if ti.ggml_type != 0:
+        raise GgufError(f"rope_freqs.weight: expected F32, got {ti.type_name}")
+    if ti.shape != (head_dim // 2,):
+        raise GgufError(f"rope_freqs.weight: shape {ti.shape} != ({head_dim // 2},) (head_dim / 2)")
+    f = g.tensor_bytes("rope_freqs.weight").view(np.float32)
+    if not (np.all(np.isfinite(f)) and np.all(f > 0)):
+        raise GgufError("rope_freqs.weight: factors must be finite and positive")
+    return tuple(float(x) for x in f)
+
+
 def _to_f32(g: Gguf, name: str) -> np.ndarray:
     ti = g.tensor_info(name)
     raw = g.tensor_bytes(name)
@@ -294,7 +308,8 @@ def host_model_from_gguf(g: Gguf, client=None):
     rows permuted for the adjacent-pair RoPE the attention operator applies) -- with any ggml weight type the library
     has a kernel for.  Anything else raises (no silent fallback): other architectures (qwen2 / phi3 / gemma use the
     NEOX rotate-half RoPE and projection biases), and files holding tensors this decoder would silently ignore
-    (*.bias, rope_freqs, stacked *_exps expert tensors -- the latter go through moe_mlp_from_gguf).
+    (*.bias, stacked *_exps expert tensors -- the latter go through moe_mlp_from_gguf).  The one optional tensor is the
+    Llama 3.1 / 3.2 rope_freqs.weight (architecture "llama" only; rope_freq_factors below).
     A quantized token_embd is dequantized on the GPU through `client`."""
     from . import synth
     from .decode import HostLinear, HostModel
@@ -306,6 +321,9 @@ def host_model_from_gguf(g: Gguf, client=None):
     cfg = config_from_gguf_metadata(g)
     names = set(g.tensor_names())
     consumed = {"token_embd.weight", "output_norm.weight", "output.weight"}
+    if arch == "llama" and "rope_freqs.weight" in names:
+        cfg.rope_freq_factors = rope_freq_factors(g, cfg.head_dim)
+        consumed.add("rope_freqs.weight")
     for i in range(cfg.n_layers):
         consumed |= {f"blk.{i}.{n}.weight" for n in ("attn_q", "attn_k", "attn_v", "attn_output", "ffn_gate", "ffn_up", "ffn_down", "attn_norm", "ffn_norm")}
     extra = sorted(names - consumed)

@@ -54,6 +54,7 @@ EXPORTS = [
     "b200q_weight_set_bias", "b200q_weight_set_next", "b200q_weight_set_pair", "b200q_shard_range", "b200q_shard_range_blocks", "b200q_workspace_bytes", "b200q_matmul",
     "b200q_act_bytes", "b200q_quantize_act", "b200q_matmul_q8", "b200q_matmul_path", "b200q_dequantize", "b200q_act_unpack",
     "b200q_int_partials", "b200q_launch_count", "b200q_add_rmsnorm_quant", "b200q_swiglu_quant", "b200q_attn_decode", "b200q_attn_decode_paged",
+    "b200q_attn_decode_max_ctx", "b200q_attn_split_workspace_bytes", "b200q_attn_decode_split", "b200q_attn_decode_paged_split",
     "b200q_argmax", "b200q_decode_error", "b200q_embed", "b200q_weight_prefetch_l2", "b200q_matmul_norm", "b200q_matmul_swiglu",
     "b200q_swiglu_f32", "b200q_swiglu_f32_interleaved", "b200q_gate_up_row", "b200q_matmul_q8_swiglu", "b200q_matmul_norm_swiglu", "b200q_moe_matmul_q8_swiglu", "b200q_program_create", "b200q_program_add_normq", "b200q_program_add_matvec", "b200q_program_add_swigluq", "b200q_program_add_attn", "b200q_program_add_argmax", "b200q_program_add_embed",
     "b200q_program_finalize", "b200q_program_launch", "b200q_program_free", "b200q_comm_create", "b200q_comm_handle", "b200q_comm_connect", "b200q_allreduce_f64", "b200q_comm_free", "b200q_comm_gather_ptr",
@@ -83,6 +84,9 @@ def lib() -> C.CDLL:
         L.b200q_weight_set_next.argtypes = [C.c_void_p, C.c_void_p]
         L.b200q_gate_up_row.restype = C.c_int64
         L.b200q_gate_up_row.argtypes = [C.c_int64, C.c_int64]
+        L.b200q_attn_decode_max_ctx.restype = C.c_int32
+        L.b200q_attn_split_workspace_bytes.restype = C.c_size_t
+        L.b200q_attn_split_workspace_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int64]
         _lib = L
     return _lib
 

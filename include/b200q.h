@@ -301,6 +301,24 @@ int32_t b200q_attn_decode(const float* qkv, const int32_t* pos, float* cache_k, 
 int32_t b200q_attn_decode_paged(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
                                 int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
                                 int64_t M, void* xq, float* attn_out, void* stream);
+/* Largest max_ctx b200q_attn_decode / b200q_attn_decode_paged accept (40960): their one CTA per (head, sequence) keeps every
+ * score of the context in shared memory.  Beyond it, use the split-context forms below. */
+int32_t b200q_attn_decode_max_ctx(void);
+/* Workspace the split-context forms need for this shape (0 for a head_dim other than 64 / 128 or non-positive sizes):
+ * f32 scores [M][nh][max_ctx] plus per-split maxima and f64 partial sums.  One workspace serves every layer of a model whose
+ * attention calls run in sequence on one stream. */
+size_t b200q_attn_split_workspace_bytes(int32_t n_heads, int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M);
+/* Split-context decode attention for any max_ctx >= 1: the arguments and results of b200q_attn_decode / _paged, computed by
+ * three kernels that split the positions of each (kv head, sequence) over up to 128 CTAs, each serving all query heads of its kv
+ * head.  Scores are bit-identical to the single-CTA kernel's; only the order of the f64 sums of the weighted sum differs.
+ * Launch shape depends on max_ctx only (graph-capturable).  A short workspace -> B200Q_ERR_WORKSPACE.  Out-of-range positions
+ * and slot -1 write nothing and raise b200q_decode_error, as in the single-CTA forms. */
+int32_t b200q_attn_decode_split(const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table, int32_t n_heads,
+                                int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* workspace,
+                                size_t workspace_bytes, void* stream);
+int32_t b200q_attn_decode_paged_split(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
+                                      int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
+                                      int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes, void* stream);
 /* A position pos[m] outside [0, max_ctx) makes b200q_attn_decode write nothing and raise a sticky per-device error
  * word instead of indexing past the KV cache.  b200q_decode_error reads and clears it for the current device
  * (synchronises the device: not capturable; call it after a generate loop).  bit 0 = position out of range. */
