@@ -657,12 +657,6 @@ int32_t b200q_matmul_swiglu(const b200q_weight* w, const float* gate_up, int64_t
     return B200Q_OK;
 }
 
-int32_t b200q_weight_prefetch_l2(const b200q_weight* w, int64_t M, int64_t max_bytes, void* stream) {
-    if (!w || max_bytes < 0) return fail(B200Q_ERR_INVALID_ARG, "bad prefetch arguments");
-    CUDA_TRY(launch_l2_prefetch(w, M, max_bytes, (cudaStream_t)stream));
-    return B200Q_OK;
-}
-
 /* debug only (not in b200q.h): per-CTA globaltimer trace of the matvec kernel */
 int32_t b200q_debug_set_matvec_trace(void* dev_buf) {
     set_matvec_trace((long long*)dev_buf);

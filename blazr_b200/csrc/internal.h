@@ -64,7 +64,6 @@ struct FusedPrologue {
 cudaError_t matvec_plan(const b200q_weight* w, int64_t M, MatvecPlan* plan, int pro = 0);
 size_t matvec_ws_bytes(const b200q_weight* w, int64_t M);  // counters + partials (excludes the activation buffer)
 void set_matvec_trace(long long* dev_buf);
-cudaError_t launch_l2_prefetch(const b200q_weight* w, int64_t M, int64_t max_bytes, cudaStream_t st);
 struct RemoteOut;  // fused TP exchange target (comm_dev.cuh: mode + CommDev)
 cudaError_t launch_matvec(const b200q_weight* w, const uint8_t* xq, int64_t M, void* y, int y_dtype, int64_t ldy, uint8_t* ws, cudaStream_t st,
                           const FusedPrologue* fp = nullptr, const RemoteOut* ro = nullptr, void* swiglu_xq_out = nullptr);

@@ -1,34 +1,10 @@
-// matvec.cu -- host side of the decode matvec: launch plan, workspace sizing, per-format dispatch, L2 prefetch hint.
+// matvec.cu -- host side of the decode matvec: launch plan, workspace sizing, per-format dispatch.
 // The kernel lives in matvec_impl.cuh and is instantiated per format in inst_<format>.cu.
 #include <cstdlib>
 
 #include "matvec_common.cuh"
 
 namespace b200q {
-
-// ------------------------------------------------------------------------------------------------
-// L2 prefetch of the chunks a following matvec launch will stream first.  The matvec CTAs own a whole SM, so
-// the next launch cannot be co-resident; instead this tiny kernel (PDL: starts as soon as the running matvec
-// releases SMs, never waits) asks the TMA engine to pull the first `nchunks` chunks of every CTA's range
-// -- in that CTA's processing order -- into L2 while the glue operators between the two matvecs run.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(32) l2_prefetch_kernel(const uint8_t* __restrict__ w, int64_t KC, int64_t C, int chunk_bytes, int first, int nchunks) {
-    pdl_launch_dependents();
-    if (threadIdx.x != 0) return;
-    const int64_t G = gridDim.x, g = blockIdx.x;
-    const int64_t c0 = sk_begin(g, C, G), c1 = sk_begin(g + 1, C, G);
-    const SkPlan sp = sk_plan(c0, c1, KC);
-    const int n = (int)(c1 - c0);
-    const uint8_t* base = w + c0 * (int64_t)chunk_bytes;
-    for (int j = first; j < n && j < first + nchunks; j++) {
-        const uint8_t* src;
-        if (j < sp.nH) src = base + (size_t)j * chunk_bytes;
-        else if (j < sp.nH + sp.nT) src = base + (size_t)(sp.nH + sp.nF + (j - sp.nH)) * chunk_bytes;
-        else src = base + (size_t)(sp.nH + (j - sp.nH - sp.nT)) * chunk_bytes;
-        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(chunk_bytes) : "memory");
-    }
-}
-
 
 static cudaError_t launch_family(int family, const MatvecParams& p, int mb, int grid, int smem, cudaStream_t st) {
     switch (family) {
@@ -235,26 +211,4 @@ cudaError_t launch_matvec_grouped(const b200q_bank* b, const int32_t* sel_dev, i
     return launch_family(v.family, p, 1, plan.grid, plan.smem_bytes, st);
 }
 
-}  // namespace b200q
-
-namespace b200q {
-cudaError_t launch_l2_prefetch(const b200q_weight* w, int64_t M, int64_t max_bytes, cudaStream_t st) {
-    MatvecPlan plan;
-    cudaError_t e = matvec_plan(w, M < 1 ? 1 : (M > 4 ? 4 : M), &plan, 0);
-    if (e != cudaSuccess) return e;
-    int nchunks = (int)(max_bytes / ((int64_t)plan.grid * w->chunk_bytes));
-    if (nchunks < 1) return cudaSuccess;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)plan.grid);
-    cfg.blockDim = dim3(32);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, l2_prefetch_kernel, (const uint8_t*)w->data, (int64_t)w->KC, (int64_t)(w->T * w->KC), w->chunk_bytes, 0, nchunks);
-    count_launch();
-    return e;
-}
 }  // namespace b200q

@@ -228,8 +228,7 @@ class Decoder:
         # fused SwiGLU epilogue (b200q_matmul_q8_swiglu): gate|up rows interleaved per tile at upload, the gate|up matvec writes the
         # down projection's activation records itself -- one launch and one kernel boundary less per layer.  ggml formats only
         # (the INT4 layouts pack 8 output rows per word), gate and up of one format, F % 64 == 0.
-        dstep = _os.environ.get("B200Q_DSTEP", "0") != "0"   # experimental op-list kernel: keeps the separate operators
-        self.swiglu_epi_wanted = ((not self.wide) and _os.environ.get("B200Q_SWIGLU_EPI", "1") != "0" and self.ff % 64 == 0 and not dstep
+        self.swiglu_epi_wanted = ((not self.wide) and _os.environ.get("B200Q_SWIGLU_EPI", "1") != "0" and self.ff % 64 == 0
                                   and _os.environ.get("B200Q_FUSED_SWIGLU", "0") == "0")
         for i in range(cfg.n_layers):
             # formats come from the weights themselves when a host model (tests, GGUF files) is given
@@ -243,7 +242,7 @@ class Decoder:
             # dual-format launch (b200q_weight_set_pair) instead of two; the tcgen05 paths keep the separate launches
             lay["qkv_mv"] = lay["qkv"]
             qk = lay["qkv"]
-            if (len(qk) == 2 and not self.wide and not dstep and _os.environ.get("B200Q_DUAL", "1") != "0" and qk[0].w.N % 128 == 0
+            if (len(qk) == 2 and not self.wide and _os.environ.get("B200Q_DUAL", "1") != "0" and qk[0].w.N % 128 == 0
                     and (qk[0].fmt, qk[1].fmt) == ("Q4_K", "Q6_K")):
                 qk[0].w.set_pair(qk[1].w)
                 lay["qkv_mv"] = [qk[0]]
@@ -272,9 +271,6 @@ class Decoder:
         self.attn_split = max_ctx > int(ops.lib().b200q_attn_decode_max_ctx())
         self.attn_ws = None
         if self.attn_split:
-            if dstep:
-                raise ValueError(f"max_ctx={max_ctx} exceeds the op-list kernel's attention limit "
-                                 f"({int(ops.lib().b200q_attn_decode_max_ctx())}): unset B200Q_DSTEP")
             nbytes = int(ops.lib().b200q_attn_split_workspace_bytes(self.nh, self.nkv, hd, max_ctx, M))
             if nbytes == 0:
                 raise ValueError(f"split-context attention does not support head_dim {hd}")
@@ -332,25 +328,16 @@ class Decoder:
         # SLOWER on the TP8 shard (3.81 vs 3.50 ms): the per-CTA norm prologue (3.6 us) costs more than the cluster kernel saves.
         self.tp_finish = tp_world > 1 and _os.environ.get("B200Q_TP_FINISH", "0") != "0" and _os.environ.get("B200Q_TP_NCCL", "0") == "0"
         self.fused = (_os.environ.get("B200Q_FUSED", "1") != "0" and not self.wide and (tp_world == 1 or self.tp_finish) and H % 512 == 0 and ept <= 16
-                      and (ept & (ept - 1)) == 0 and not dstep)
+                      and (ept & (ept - 1)) == 0)
         self.tp_finish = self.tp_finish and self.fused
         self.fused_swiglu = _os.environ.get("B200Q_FUSED_SWIGLU", "0") != "0" and not self.wide  # measured slower: 148x redundant SiLU
-        self.pf_bytes = int(float(_os.environ.get("B200Q_PF_MB", "0")) * (1 << 20))
         self.graph = None
         self._host_pos = 0
-        # EXPERIMENTAL (B200Q_DSTEP=1, single GPU, M <= 4): persistent op-list kernel, 3 launches per layer instead of 8
-        self.programs = None
-        self.step_program = None
-        if _os.environ.get("B200Q_DSTEP", "0") != "0" and tp_world == 1 and not self.wide and not self.fused:
-            if _os.environ.get("B200Q_DSTEP") == "2":
-                self._build_step_program()
-            else:
-                self._build_programs()
         # tensor parallel: one-shot NVLink all-reduce of the f64 partial sums (csrc/comm.cu); B200Q_TP_NCCL=1 falls back
         # to torch.distributed (NCCL) all-reduce of f32 partials for comparison
         self.comm = None
         if tp_world > 1 and _os.environ.get("B200Q_TP_NCCL", "0") == "0":
-            assert (self.tp_finish or not self.fused) and not self.fused_swiglu and self.programs is None and self.step_program is None
+            assert (self.tp_finish or not self.fused) and not self.fused_swiglu
             self.vs = tp.vocab_shard_rows(cfg.vocab, tp_world)
             if emulate_shard:
                 self.comm = ops.PeerComm(0, 1, M * H, dev, None, gather_elems=M * self.vs)
@@ -431,87 +418,7 @@ class Decoder:
             return self.c.weight_from_decomposed(dq)
         raise ValueError(fmt)
 
-    def _build_step_program(self):
-        """B200Q_DSTEP=2: the WHOLE step as one program / one launch (embed ... argmax), attention included"""
-        cfg, M = self.cfg, self.M
-        pr = ops.Program(self.dev)
-        pr.embed(self.embed, self.ids, self.h)
-        hin, hout = self.h, self.h2
-        delta = None
-        for lay in self.layers:
-            pr.normq(hin, delta, hout, lay["attn_norm"], cfg.eps, self.xq_h)
-            hin, hout = hout, hin
-            for ln in lay["qkv"]:
-                pr.matvec(ln.w, self.xq_h, M, self.qkv, ln.col0, ln.ws)
-            pr.attn(self.qkv, self.pos, lay["ck"], lay["cv"], self.rope, self.nh, self.nkv, cfg.head_dim, self.max_ctx, M, self.xq_attn)
-            for ln in lay["o"]:
-                pr.matvec(ln.w, self.xq_attn, M, self.delta, ln.col0, ln.ws)
-            pr.normq(hin, self.delta, hout, lay["mlp_norm"], cfg.eps, self.xq_h)
-            hin, hout = hout, hin
-            for ln in lay["gu"]:
-                pr.matvec(ln.w, self.xq_h, M, self.gu, ln.col0, ln.ws)
-            pr.swigluq(self.gu, self.ff, M, self.xq_ff)
-            for ln in lay["down"]:
-                pr.matvec(ln.w, self.xq_ff, M, self.delta2, ln.col0, ln.ws)
-            delta = self.delta2
-        pr.normq(hin, delta, hout, self.final_norm, cfg.eps, self.xq_h)
-        for ln in self.head:
-            pr.matvec(ln.w, self.xq_h, M, self.logits_local, ln.col0, ln.ws)
-        pr.argmax(self.logits, self.ids, self.pos)
-        self.step_program = pr.finalize()
-
-    def _build_programs(self):
-        """op lists between the attention operators of a step (same buffers and order as step())"""
-        cfg, M = self.cfg, self.M
-        progs = []
-        hin, hout = self.h, self.h2
-        delta = None
-        for lay in self.layers:
-            p1 = ops.Program(self.dev)
-            p1.normq(hin, delta, hout, lay["attn_norm"], cfg.eps, self.xq_h)
-            hin, hout = hout, hin
-            for ln in lay["qkv"]:
-                p1.matvec(ln.w, self.xq_h, M, self.qkv, ln.col0, ln.ws)
-            p2 = ops.Program(self.dev)
-            for ln in lay["o"]:
-                p2.matvec(ln.w, self.xq_attn, M, self.delta, ln.col0, ln.ws)
-            p2.normq(hin, self.delta, hout, lay["mlp_norm"], cfg.eps, self.xq_h)
-            hin, hout = hout, hin
-            for ln in lay["gu"]:
-                p2.matvec(ln.w, self.xq_h, M, self.gu, ln.col0, ln.ws)
-            p2.swigluq(self.gu, self.ff, M, self.xq_ff)
-            for ln in lay["down"]:
-                p2.matvec(ln.w, self.xq_ff, M, self.delta2, ln.col0, ln.ws)
-            delta = self.delta2
-            progs.append((p1.finalize(), p2.finalize()))
-        pf = ops.Program(self.dev)
-        pf.normq(hin, delta, hout, self.final_norm, cfg.eps, self.xq_h)
-        for ln in self.head:
-            pf.matvec(ln.w, self.xq_h, M, self.logits_local, ln.col0, ln.ws)
-        self.programs = (progs, pf.finalize())
-
-    def _step_programs(self):
-        L, cfg, M = ops.lib(), self.cfg, self.M
-        st = ops._stream_ptr(self.dev)
-        P = lambda t: C.c_void_p(t.data_ptr())
-        ops._check(L.b200q_embed(P(self.embed), P(self.ids), C.c_int64(cfg.hidden), C.c_int64(M), P(self.h), st))
-        progs, pf = self.programs
-        for lay, (p1, p2) in zip(self.layers, progs):
-            p1.launch()
-            ops._check(L.b200q_attn_decode(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.rope), C.c_int32(self.nh),
-                                           C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M),
-                                           P(self.xq_attn), None, st))
-            p2.launch()
-        pf.launch()
-        ops._check(L.b200q_argmax(P(self.logits), C.c_int64(self.logits.shape[1]), C.c_int64(M), P(self.ids), P(self.pos), st))
-
     # ---- one decode step ------------------------------------------------------------------------------
-    def _prefetch(self, lins: List[_Linear]):
-        """L2 prefetch hint for the matvec that follows the upcoming glue operator"""
-        if self.pf_bytes <= 0:
-            return
-        ops._check(ops.lib().b200q_weight_prefetch_l2(lins[0].w.handle, C.c_int64(self.M), C.c_int64(self.pf_bytes), ops._stream_ptr(self.dev)))
-
     def _matvec(self, lins: List[_Linear], xq: torch.Tensor, out: torch.Tensor):
         L = ops.lib()
         st = ops._stream_ptr(self.dev)
@@ -620,10 +527,6 @@ class Decoder:
         """ids (device) -> next ids (device); positions advance on the device: graph-replayable."""
         if not torch.cuda.is_current_stream_capturing():
             self._advance()
-        if self.step_program is not None:
-            return self.step_program.launch()
-        if self.programs is not None:
-            return self._step_programs()
         L, cfg, M = ops.lib(), self.cfg, self.M
         st = ops._stream_ptr(self.dev)
         P = lambda t: C.c_void_p(t.data_ptr())

@@ -55,9 +55,9 @@ EXPORTS = [
     "b200q_act_bytes", "b200q_quantize_act", "b200q_matmul_q8", "b200q_matmul_path", "b200q_dequantize", "b200q_act_unpack",
     "b200q_int_partials", "b200q_launch_count", "b200q_add_rmsnorm_quant", "b200q_swiglu_quant", "b200q_attn_decode", "b200q_attn_decode_paged",
     "b200q_attn_decode_max_ctx", "b200q_attn_split_workspace_bytes", "b200q_attn_decode_split", "b200q_attn_decode_paged_split",
-    "b200q_argmax", "b200q_decode_error", "b200q_embed", "b200q_weight_prefetch_l2", "b200q_matmul_norm", "b200q_matmul_swiglu",
-    "b200q_swiglu_f32", "b200q_swiglu_f32_interleaved", "b200q_gate_up_row", "b200q_matmul_q8_swiglu", "b200q_matmul_norm_swiglu", "b200q_moe_matmul_q8_swiglu", "b200q_program_create", "b200q_program_add_normq", "b200q_program_add_matvec", "b200q_program_add_swigluq", "b200q_program_add_attn", "b200q_program_add_argmax", "b200q_program_add_embed",
-    "b200q_program_finalize", "b200q_program_launch", "b200q_program_free", "b200q_comm_create", "b200q_comm_handle", "b200q_comm_connect", "b200q_allreduce_f64", "b200q_comm_free", "b200q_comm_gather_ptr",
+    "b200q_argmax", "b200q_decode_error", "b200q_embed", "b200q_matmul_norm", "b200q_matmul_swiglu",
+    "b200q_swiglu_f32", "b200q_swiglu_f32_interleaved", "b200q_gate_up_row", "b200q_matmul_q8_swiglu", "b200q_matmul_norm_swiglu", "b200q_moe_matmul_q8_swiglu",
+    "b200q_comm_create", "b200q_comm_handle", "b200q_comm_connect", "b200q_allreduce_f64", "b200q_comm_free", "b200q_comm_gather_ptr",
     "b200q_matmul_q8_rowpar", "b200q_allreduce_add_rmsnorm_quant", "b200q_allreduce_finish", "b200q_matmul_q8_gather", "b200q_argmax_gathered", "b200q_allreduce",
     "b200q_bank_create", "b200q_bank_free", "b200q_bank_set", "b200q_bank_get", "b200q_bank_workspace_bytes", "b200q_moe_matmul_q8", "b200q_moe_combine",
 ]
@@ -442,66 +442,6 @@ class MoeMlp:
                                      C.c_int64(self.hidden), P(b["ws_dn"]), C.c_size_t(b["ws_dn"].numel()), st))
         _check(L.b200q_moe_combine(P(b["y"]), P(gw), C.c_int64(T), C.c_int64(top_k), C.c_int64(self.hidden), P(b["out"]), st))
         return b["out"]
-
-
-class Program:
-    """EXPERIMENTAL: op list for the persistent kernel (include/b200q.h b200q_program_*).  Buffers must stay alive and at
-    the same addresses for the life of the program (the decode harness allocates them once)."""
-
-    def __init__(self, device: torch.device):
-        self.device = device
-        h = C.c_void_p()
-        _check(lib().b200q_program_create(C.c_int32(device.index or 0), C.byref(h)))
-        self._h = h
-        self.n_ops = 0
-
-    def normq(self, h_in, delta, h_out, norm_w, eps: float, xq_out):
-        M, H = h_in.shape
-        _check(lib().b200q_program_add_normq(self._h, C.c_void_p(h_in.data_ptr()), C.c_void_p(delta.data_ptr()) if delta is not None else None,
-                                             C.c_void_p(h_out.data_ptr()), C.c_void_p(norm_w.data_ptr()), C.c_float(eps), C.c_int64(H), C.c_int64(M),
-                                             C.c_void_p(xq_out.data_ptr())))
-        self.n_ops += 1
-
-    def matvec(self, w: QuantWeight, xq, M: int, out, col0: int, ws):
-        dt = F64 if out.dtype == torch.float64 else F32
-        _check(lib().b200q_program_add_matvec(self._h, w.handle, C.c_void_p(xq.data_ptr()), C.c_int64(M),
-                                              C.c_void_p(out.data_ptr() + out.element_size() * col0), C.c_int32(dt), C.c_int64(out.stride(0)),
-                                              C.c_void_p(ws.data_ptr()), C.c_size_t(ws.numel())))
-        self.n_ops += 1
-
-    def swigluq(self, gate_up, F_: int, M: int, xq_out):
-        _check(lib().b200q_program_add_swigluq(self._h, C.c_void_p(gate_up.data_ptr()), C.c_int64(F_), C.c_int64(M), C.c_void_p(xq_out.data_ptr())))
-        self.n_ops += 1
-
-    def attn(self, qkv, pos, ck, cv, rope, nh: int, nkv: int, hd: int, max_ctx: int, M: int, xq_out):
-        _check(lib().b200q_program_add_attn(self._h, C.c_void_p(qkv.data_ptr()), C.c_void_p(pos.data_ptr()), C.c_void_p(ck.data_ptr()),
-                                            C.c_void_p(cv.data_ptr()), C.c_void_p(rope.data_ptr()), C.c_int32(nh), C.c_int32(nkv), C.c_int32(hd),
-                                            C.c_int32(max_ctx), C.c_int64(M), C.c_void_p(xq_out.data_ptr())))
-        self.n_ops += 1
-
-    def argmax(self, logits, ids, pos):
-        M, V = logits.shape
-        _check(lib().b200q_program_add_argmax(self._h, C.c_void_p(logits.data_ptr()), C.c_int64(V), C.c_int64(M), C.c_void_p(ids.data_ptr()),
-                                              C.c_void_p(pos.data_ptr())))
-        self.n_ops += 2
-
-    def embed(self, table, ids, h):
-        M, H = h.shape
-        _check(lib().b200q_program_add_embed(self._h, C.c_void_p(table.data_ptr()), C.c_void_p(ids.data_ptr()), C.c_int64(H), C.c_int64(M),
-                                             C.c_void_p(h.data_ptr())))
-        self.n_ops += 1
-
-    def finalize(self):
-        _check(lib().b200q_program_finalize(self._h))
-        return self
-
-    def launch(self):
-        _check(lib().b200q_program_launch(self._h, _stream_ptr(self.device)))
-
-    def free(self):
-        if self._h is not None:
-            lib().b200q_program_free(self._h)
-            self._h = None
 
 
 class _DevView:

@@ -157,25 +157,6 @@ int32_t b200q_quantize_act(const void* x, int32_t x_dtype, int64_t M, int64_t K,
                            void* xq, void* stream);
 int32_t b200q_matmul_q8(const b200q_weight* w, const void* xq, int64_t M, void* y, int32_t y_dtype, int64_t ldy,
                         void* workspace, size_t workspace_bytes, void* stream);
-/* ---- EXPERIMENTAL persistent op-list kernel (csrc/dstep_impl.cuh; opt-in, not yet run on hardware) ----
- * A program is a list of ops executed by ONE launch of one CTA per SM, separated by grid barriers, while the weight
- * stream of all its matvecs runs ahead of the dependencies: normq = b200q_add_rmsnorm_quant, matvec = b200q_matmul_q8
- * (M in {1,2,4}, Q4_K / Q6_K / Q8_0 / AWQ-GPTQ), swigluq = b200q_swiglu_quant, with identical arithmetic.  Replaces the
- * separate launches between two attention operators of a decode step (reference call pattern: cuda_graphs.rs:101-189). */
-typedef struct b200q_program b200q_program;
-int32_t b200q_program_create(int32_t device, b200q_program** out);
-int32_t b200q_program_add_normq(b200q_program* p, const float* h_in, const float* delta, float* h_out, const float* norm_w, float eps,
-                                int64_t H, int64_t M, void* xq_out);
-int32_t b200q_program_add_matvec(b200q_program* p, const b200q_weight* w, const void* xq, int64_t M, void* y, int32_t y_dtype, int64_t ldy,
-                                 void* workspace, size_t workspace_bytes);
-int32_t b200q_program_add_swigluq(b200q_program* p, const float* gate_up, int64_t F, int64_t M, void* xq_out);
-int32_t b200q_program_add_attn(b200q_program* p, const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table,
-                               int32_t n_heads, int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq_out);
-int32_t b200q_program_add_argmax(b200q_program* p, const float* logits, int64_t V, int64_t M, int64_t* out_ids, int32_t* pos_inc);
-int32_t b200q_program_add_embed(b200q_program* p, const void* table_f16, const int64_t* ids, int64_t H, int64_t M, float* h);
-int32_t b200q_program_finalize(b200q_program* p);
-int32_t b200q_program_launch(const b200q_program* p, void* stream);
-int32_t b200q_program_free(b200q_program* p);
 
 /* ---- expert banks (MoE): reference boostr::ExpertWeights{gate_proj, up_proj, down_proj}, stacked
  * [num_experts, dim_in, dim_out] and sliced per expert (src/engine/executor_cache.rs:19,218-228,260,283,344-348).
@@ -257,9 +238,6 @@ int32_t b200q_matmul_norm_swiglu(const b200q_weight* w, const float* h_in, const
                                  void* xq_out, void* workspace, size_t workspace_bytes, void* stream);
 int32_t b200q_moe_matmul_q8_swiglu(const b200q_bank* b, const int32_t* sel_dev, int64_t n_slots, const void* xq, int64_t x_rows, int64_t x_slot_div,
                                    void* xq_out, void* workspace, size_t workspace_bytes, void* stream);
-/* Hint: ask the TMA engine to pull the first `max_bytes` of w (in the order the next b200q_matmul_q8(w, M) will
- * stream them) into L2.  Enqueue it right after the preceding matmul: it overlaps the operators in between. */
-int32_t b200q_weight_prefetch_l2(const b200q_weight* w, int64_t M, int64_t max_bytes, void* stream);
 /* Force a path (testing / benchmarking): 0 = auto, 1 = dp4a matvec, 2 = tcgen05 GEMM */
 int32_t b200q_matmul_path(const b200q_weight* w, int32_t path, const void* x, int32_t x_dtype, int64_t M, int64_t ldx, void* y,
                           int32_t y_dtype, int64_t ldy, void* workspace, size_t workspace_bytes, void* stream);
