@@ -43,20 +43,18 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 }
 
 // raw 32-bit shared-window addresses (computed once outside hot loops: no per-iteration cvta)
-__device__ __forceinline__ void mbar_wait_sa(uint32_t bar_sa, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(bar_sa), "r"(parity)
-            : "memory");
-    } while (!ok);
-}
 __device__ __forceinline__ void mbar_arrive_sa(uint32_t bar_sa) {
     asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(bar_sa) : "memory");
+}
+// the retry loop stays inside one asm statement: no compiler-built loop (and convergence region) around a per-lane flag
+__device__ __forceinline__ void mbar_wait_sa(uint32_t bar_sa, uint32_t parity) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n"
+        "MBAR_WAIT:\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
+        "@!p bra MBAR_WAIT;\n\t}" ::"r"(bar_sa),
+        "r"(parity)
+        : "memory");
 }
 
 // ---- bulk async copy global -> shared (TMA engine, 1-D), completion on an mbarrier ----
@@ -168,6 +166,16 @@ __device__ __forceinline__ uint32_t keep_in_reg(uint32_t v) {
 }
 
 __device__ __forceinline__ float half_bits_to_float(uint16_t h) { return __half2float(__ushort_as_half(h)); }
+// (f16 in the low or high half of hw) x (f16 in the low half of q), one rounding to f32 (sm_100 FHFMA); with q = an integer
+// n < 1024 as f16 bits (the subnormal n * 2^-24) the result is h * n * 2^-24, exact whenever h * n has <= 24 significant bits
+template <int HALF>
+__device__ __forceinline__ float fma_f16_f32(uint32_t hw, uint32_t q) {
+    uint16_t lo, hi;
+    asm("mov.b32 {%0,%1}, %2;" : "=h"(lo), "=h"(hi) : "r"(hw));
+    float r;
+    asm("fma.rn.f32.f16 %0, %1, %2, %3;" : "=f"(r) : "h"(HALF ? hi : lo), "h"((uint16_t)q), "f"(-0.0f));
+    return r;
+}
 
 // dtype codes mirror b200q_dtype
 template <typename T>

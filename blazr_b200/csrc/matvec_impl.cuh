@@ -294,6 +294,8 @@ __global__ void __launch_bounds__(MV_THREADS, 1) matvec_kernel(const MatvecParam
     constexpr bool RP = OUT == OUT_REMOTE;
     constexpr bool EPI = OUT == OUT_SWIGLU;
     constexpr bool DUAL = !std::is_same<F, F2>::value;   // two weights of different formats in one grid (MatvecParams::w2)
+    // M = 1: two chunks per trip of the consumer loop (one counter test and branch per pair); the M = 2 / 4 loops would spill
+    constexpr int MV_CHUNK_UNROLL = MB == 1 ? 2 : 1;
     static_assert(!DUAL || (!GRP && OUT == OUT_PLAIN), "the dual-format launch is a plain matvec");
     __shared__ float s_y[EPI ? 2 : 1][EPI ? MB : 1][EPI ? TILE_ROWS : 1];   // finished full tiles (double-buffered)
     __shared__ float s_yfix[EPI ? MB : 1][EPI ? TILE_ROWS : 1];             // finished split tile (fix-up warp only)
@@ -595,7 +597,6 @@ __global__ void __launch_bounds__(MV_THREADS, 1) matvec_kernel(const MatvecParam
     int seg = sp.nH > 0 ? 0 : (sp.nT > 0 ? 1 : 2);
     int seg_left = seg == 0 ? sp.nH : (seg == 1 ? sp.nT : KC);  // chunks until the next flush
     int t = seg == 0 ? sp.tH : (seg == 1 ? sp.tT : sp.tF);
-    int s = 0;
     uint32_t ph = 0;
     int n_full_done = 0;  // OUT_SWIGLU: full tiles flushed so far (selects the s_y buffer)
     // Everything the hot loop addresses is a 32-bit shared-window address built from values computed ONCE here: the ring /
@@ -604,7 +605,7 @@ __global__ void __launch_bounds__(MV_THREADS, 1) matvec_kernel(const MatvecParam
     constexpr int NOFF = FmtNoff<F>::value;
     const uint32_t stages_sa = smem_u32(stages), full_sa = keep_in_reg(smem_u32(full)), xhat_sa = smem_u32(xhat);
     constexpr uint32_t EMPTY_OFF = MV_MAX_STAGES * 8;                     // empty[] follows full[]
-    const uint32_t ring_bytes = (uint32_t)nst * (uint32_t)p.stage_bytes;
+    const uint32_t ring_bytes = keep_in_reg((uint32_t)nst * (uint32_t)p.stage_bytes);
     uint32_t st_off = 0;                                                   // byte offset of stage s inside the ring
     uint32_t bar_sa = full_sa;                                             // full[s]; empty[s] = + EMPTY_OFF
     uint32_t uoff[NOFF > 0 ? NOFF : 1];
@@ -623,87 +624,91 @@ __global__ void __launch_bounds__(MV_THREADS, 1) matvec_kernel(const MatvecParam
     }
     const uint32_t xq_off = keep_in_reg((PRO ? xhat_sa : stages_sa + (uint32_t)p.chunk_bytes) + 32u * (uint32_t)i);      // int8 activations of unit i
     const uint32_t xs_off = keep_in_reg((PRO ? xhat_sa : stages_sa + (uint32_t)p.chunk_bytes) + 256u + 4u * (uint32_t)i); // its scale; + 32: block sums
-    const uint32_t xrec_step = (uint32_t)p.M * ACT_REC_BYTES;
+    const uint32_t xrec_step = keep_in_reg((uint32_t)p.M * ACT_REC_BYTES);
+    const uint32_t stage_bytes = keep_in_reg((uint32_t)p.stage_bytes);
     uint32_t xk_off = PRO ? (uint32_t)kcur * xrec_step : 0u;               // PRO: record of k-chunk kcur inside xhat
-    for (int j = 0; j < n_chunks; j++) {
-        mbar_wait_sa(bar_sa, ph);
-        if (MV_TRACE_ON(p) && tid == 0 && j == 0) p.trace[g * 8 + 1] = globaltimer_ns();
-        const uint8_t* wc = stages + (size_t)s * p.stage_bytes;
-        const uint32_t xbase = PRO ? xk_off : st_off;
-        if (PRO) { xk_off += xrec_step; if (++kcur == KC) { kcur = 0; xk_off = 0u; } }
+    // one trip of the outer loop per segment; a segment never crosses a tile boundary, so kcur does not wrap inside it
+    for (int j = 0; j < n_chunks;) {
+#pragma unroll(MV_CHUNK_UNROLL)
+        for (int c = seg_left; c > 0; c--) {
+            mbar_wait_sa(bar_sa, ph);
+            if (MV_TRACE_ON(p) && tid == 0 && j == 0 && c == seg_left) p.trace[g * 8 + 1] = globaltimer_ns();
+            const uint8_t* wc = stages + st_off;
+            const uint32_t xbase = PRO ? xk_off : st_off;
+            if (PRO) xk_off += xrec_step;
 
-        uint4 xa[MB], xb[MB];
-        float dx[MB];
-        int bsA[MB], bsB[MB];
+            uint4 xa[MB], xb[MB];
+            float dx[MB];
+            int bsA[MB], bsB[MB];
 #pragma unroll
-        for (int m = 0; m < MB; m++) {
-            xa[m] = lds128_sa(xq_off + xbase + m * ACT_REC_BYTES);
-            xb[m] = lds128_sa(xq_off + xbase + m * ACT_REC_BYTES + 16);
-            dx[m] = __uint_as_float(lds32_sa(xs_off + xbase + m * ACT_REC_BYTES));
-            const uint32_t bs = lds32_sa(xs_off + xbase + m * ACT_REC_BYTES + 32);
-            bsA[m] = (int)(int16_t)(bs & 0xFFFFu);
-            bsB[m] = (int)(int16_t)(bs >> 16);
-        }
-        const bool skip_chunk = GRP && *reinterpret_cast<const volatile int*>(wc + p.chunk_bytes + p.M * ACT_REC_BYTES) != 0;
-        // the units of this chunk: rows 8 warp + 4 s4 + g4, unit i -- format FF (dual-format launches pick it per tile)
-        auto chunk_math = [&](auto tag, const auto& uo, const FmtMeta& mt) {
-            using FF = decltype(tag);
-            constexpr int NO = FmtNoff<FF>::value;
+            for (int m = 0; m < MB; m++) {
+                xa[m] = lds128_sa(xq_off + xbase + m * ACT_REC_BYTES);
+                xb[m] = lds128_sa(xq_off + xbase + m * ACT_REC_BYTES + 16);
+                dx[m] = __uint_as_float(lds32_sa(xs_off + xbase + m * ACT_REC_BYTES));
+                const uint32_t bs = lds32_sa(xs_off + xbase + m * ACT_REC_BYTES + 32);
+                bsA[m] = (int)(int16_t)(bs & 0xFFFFu);
+                bsB[m] = (int)(int16_t)(bs >> 16);
+            }
+            const bool skip_chunk = GRP && *reinterpret_cast<const volatile int*>(wc + p.chunk_bytes + p.M * ACT_REC_BYTES) != 0;
+            // the units of this chunk: rows 8 warp + 4 s4 + g4, unit i -- format FF (dual-format launches pick it per tile)
+            auto chunk_math = [&](auto tag, const auto& uo, const FmtMeta& mt) {
+                using FF = decltype(tag);
+                constexpr int NO = FmtNoff<FF>::value;
 #pragma unroll
-            for (int s4 = 0; s4 < MV_STEPS; s4++) {
-                Unit u;
-                if constexpr (NO > 0) {
-                    if (s4 == 0) FF::template load_unit_at<0>(st_off, uo, i, u, mt);
-                    else FF::template load_unit_at<1>(st_off, uo, i, u, mt);
-                } else {
-                    const int r = MV_ROWS_PER_WARP * warp + 4 * s4 + g4;
-                    FF::template load_unit<true, FF::NIB>(wc, r, i, u, mt);
-                }
-#pragma unroll
-                for (int m = 0; m < MB; m++) {
-                    int sA = 0, sB = 0;
-                    sA = __dp4a((int)u.v[0], (int)xa[m].x, sA); sA = __dp4a((int)u.v[1], (int)xa[m].y, sA);
-                    sA = __dp4a((int)u.v[2], (int)xa[m].z, sA); sA = __dp4a((int)u.v[3], (int)xa[m].w, sA);
-                    if constexpr (FF::NIB) {  // bytes hold 16 x q (unsigned): exact u8 x s8 dot, one arithmetic shift back
-                        sB = dp4a_us(u.v[4], xb[m].x, sB); sB = dp4a_us(u.v[5], xb[m].y, sB);
-                        sB = dp4a_us(u.v[6], xb[m].z, sB); sB = dp4a_us(u.v[7], xb[m].w, sB);
-                        sB >>= 4;
+                for (int s4 = 0; s4 < MV_STEPS; s4++) {
+                    Unit u;
+                    if constexpr (NO > 0) {
+                        if (s4 == 0) FF::template load_unit_at<0>(st_off, uo, i, u, mt);
+                        else FF::template load_unit_at<1>(st_off, uo, i, u, mt);
                     } else {
-                        sB = __dp4a((int)u.v[4], (int)xb[m].x, sB); sB = __dp4a((int)u.v[5], (int)xb[m].y, sB);
-                        sB = __dp4a((int)u.v[6], (int)xb[m].z, sB); sB = __dp4a((int)u.v[7], (int)xb[m].w, sB);
+                        const int r = MV_ROWS_PER_WARP * warp + 4 * s4 + g4;
+                        FF::template load_unit<true, FF::NIB>(wc, r, i, u, mt);
                     }
-                    sA -= u.off[0] * bsA[m];
-                    sB -= u.off[1] * bsB[m];
-                    double a_ = acc[s4][m];
-                    if (FF::SUB == 32) {  // one scale per 32 weights
-                        a_ = fma((double)__fmul_rn(u.a[0], dx[m]), i2d(sA + sB), a_);
-                        if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[0], dx[m]), i2d(bsA[m] + bsB[m]), a_);
-                    } else {             // two 16-wide sub-blocks with their own scales
-                        a_ = fma((double)__fmul_rn(u.a[0], dx[m]), i2d(sA), a_);
-                        if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[0], dx[m]), i2d(bsA[m]), a_);
-                        a_ = fma((double)__fmul_rn(u.a[1], dx[m]), i2d(sB), a_);
-                        if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[1], dx[m]), i2d(bsB[m]), a_);
+#pragma unroll
+                    for (int m = 0; m < MB; m++) {
+                        const float dxm = FmtAbScale<FF>::value ? __fmul_rn(dx[m], FmtAbScale<FF>::inv) : dx[m];
+                        int sA = 0, sB = 0;
+                        sA = __dp4a((int)u.v[0], (int)xa[m].x, sA); sA = __dp4a((int)u.v[1], (int)xa[m].y, sA);
+                        sA = __dp4a((int)u.v[2], (int)xa[m].z, sA); sA = __dp4a((int)u.v[3], (int)xa[m].w, sA);
+                        if constexpr (FF::NIB) {  // bytes hold 16 x q (unsigned): exact u8 x s8 dot, one arithmetic shift back
+                            sB = dp4a_us(u.v[4], xb[m].x, sB); sB = dp4a_us(u.v[5], xb[m].y, sB);
+                            sB = dp4a_us(u.v[6], xb[m].z, sB); sB = dp4a_us(u.v[7], xb[m].w, sB);
+                            sB >>= 4;
+                        } else {
+                            sB = __dp4a((int)u.v[4], (int)xb[m].x, sB); sB = __dp4a((int)u.v[5], (int)xb[m].y, sB);
+                            sB = __dp4a((int)u.v[6], (int)xb[m].z, sB); sB = __dp4a((int)u.v[7], (int)xb[m].w, sB);
+                        }
+                        sA -= u.off[0] * bsA[m];
+                        sB -= u.off[1] * bsB[m];
+                        double a_ = acc[s4][m];
+                        if (FF::SUB == 32) {  // one scale per 32 weights
+                            a_ = fma((double)__fmul_rn(u.a[0], dxm), i2d(sA + sB), a_);
+                            if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[0], dxm), i2d(bsA[m] + bsB[m]), a_);
+                        } else {             // two 16-wide sub-blocks with their own scales
+                            a_ = fma((double)__fmul_rn(u.a[0], dxm), i2d(sA), a_);
+                            if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[0], dxm), i2d(bsA[m]), a_);
+                            a_ = fma((double)__fmul_rn(u.a[1], dxm), i2d(sB), a_);
+                            if (FF::HAS_MIN) a_ = fma(-(double)__fmul_rn(u.b[1], dxm), i2d(bsB[m]), a_);
+                        }
+                        acc[s4][m] = a_;
                     }
-                    acc[s4][m] = a_;
+                }
+            };
+            if (!MV_DEBUG_SKIP(p) && !skip_chunk) {
+                if constexpr (DUAL) {
+                    if (t >= p.T1) chunk_math(F2{}, uoff2, meta2);   // warp-uniform: a tile belongs to one weight
+                    else chunk_math(F{}, uoff, meta);
+                } else {
+                    chunk_math(F{}, uoff, meta);
                 }
             }
-        };
-        if (!MV_DEBUG_SKIP(p) && !skip_chunk) {
-            if constexpr (DUAL) {
-                if (t >= p.T1) chunk_math(F2{}, uoff2, meta2);   // warp-uniform: a tile belongs to one weight
-                else chunk_math(F{}, uoff, meta);
-            } else {
-                chunk_math(F{}, uoff, meta);
-            }
+            // release the stage: the warp is converged here, so every lane's loads of it were issued before lane 0's arrive (no
+            // __syncwarp and its divergence check), and the producer's refill lands a whole HBM round trip after the arrive
+            if (lane == 0) mbar_arrive_sa(bar_sa + EMPTY_OFF);
+            st_off += stage_bytes;
+            bar_sa += 8u;
+            if (st_off == ring_bytes) { ph ^= 1u; st_off = 0u; bar_sa = full_sa; }
         }
-        __syncwarp();
-        if (lane == 0) mbar_arrive_sa(bar_sa + EMPTY_OFF);
-        st_off += (uint32_t)p.stage_bytes;
-        bar_sa += 8u;
-        ++s;
-        if (st_off == ring_bytes) { s = 0; ph ^= 1u; st_off = 0u; bar_sa = full_sa; }
-
-        if (--seg_left > 0) continue;
 
         // ---- segment / tile boundary: reduce the 8 lanes of each row and flush ----
 #pragma unroll
@@ -828,8 +833,10 @@ __global__ void __launch_bounds__(MV_THREADS, 1) matvec_kernel(const MatvecParam
             for (int m = 0; m < MB; m++) acc[s4][m] = 0.0;
 
         // ---- next segment / tile ----
-        if (seg == 0 && sp.nT > 0) { seg = 1; seg_left = sp.nT; t = sp.tT; kcur = 0; xk_off = 0u; }
-        else if (seg != 2) { seg = 2; seg_left = KC; t = sp.tF; kcur = 0; xk_off = 0u; }
+        j += seg_left;
+        xk_off = 0u;
+        if (seg == 0 && sp.nT > 0) { seg = 1; seg_left = sp.nT; t = sp.tT; }
+        else if (seg != 2) { seg = 2; seg_left = KC; t = sp.tF; }
         else { seg_left = KC; t++; }
 
     }
