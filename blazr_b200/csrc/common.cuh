@@ -100,6 +100,10 @@ __device__ __forceinline__ float det_expf(float x) {
     return __fmul_rn(p, __int_as_float(((int)n + 127) << 23));
 }
 
+// Element rule of an f16 KV cache (decode attention): f16_rn(clamp(x, +-65504)).  Finite inputs stay finite; fmaxf maps NaN
+// to -65504.  Restated by blazr_b200/decode.py kv_round (prefill writes) and tests/kv16_ref.py kv_round_np (the oracle).
+__device__ __forceinline__ __half kv_f16_rn(float x) { return __float2half_rn(fminf(fmaxf(x, -65504.0f), 65504.0f)); }
+
 // one elected lane of a converged warp (the compiler then emits tcgen05 / TMA instructions of the guarded region
 // without per-instruction uniformity loops)
 __device__ __forceinline__ bool elect_one() {

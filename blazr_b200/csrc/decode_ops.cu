@@ -7,6 +7,7 @@
 // producers before touching global memory.
 #include <cooperative_groups.h>
 #include <cstdlib>
+#include <type_traits>
 
 #include "comm_dev.cuh"
 #include "common.cuh"
@@ -281,9 +282,35 @@ struct PagedKv {
     const int* slot_mapping;  // [M] or null
     int block_size, max_blocks;
 };
-template <int HD, bool PAGED>
-__global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, float* __restrict__ cache_k,
-                                                           float* __restrict__ cache_v, const float* __restrict__ rope, int nh, int nkv,
+
+// KV cache element type T: float, or __half (kv_f16_rn on append).  Every cached value widens exactly to f32 on load, so all
+// arithmetic after the load is the same for both.  kv_line_t is one 16-byte load (4 f32 / 8 f16 elements), kv_quad_t one load
+// of 4 elements (16 / 8 bytes).
+template <typename T> using kv_line_t = std::conditional_t<std::is_same_v<T, float>, float4, uint4>;
+template <typename T> using kv_quad_t = std::conditional_t<std::is_same_v<T, float>, float4, uint2>;
+template <typename T> constexpr int KV_LINE = 16 / (int)sizeof(T);
+template <typename T> __device__ __forceinline__ kv_line_t<T> kv_ld_line(const T* p) { return *reinterpret_cast<const kv_line_t<T>*>(p); }
+template <typename T> __device__ __forceinline__ kv_quad_t<T> kv_ld_quad(const T* p) { return *reinterpret_cast<const kv_quad_t<T>*>(p); }
+template <typename T> __device__ __forceinline__ T kv_store_val(float x) {
+    if constexpr (std::is_same_v<T, float>) return x;
+    else return kv_f16_rn(x);
+}
+__device__ __forceinline__ float4 kv_widen(const float4& v) { return v; }
+__device__ __forceinline__ float4 kv_widen(const uint2& v) {
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&v.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&v.y));
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ void kv_widen(const uint4& v, float* o) {
+    const float4 a = kv_widen(make_uint2(v.x, v.y)), b = kv_widen(make_uint2(v.z, v.w));
+    o[0] = a.x; o[1] = a.y; o[2] = a.z; o[3] = a.w; o[4] = b.x; o[5] = b.y; o[6] = b.z; o[7] = b.w;
+}
+// 4 consecutive elements, widened
+template <typename T> __device__ __forceinline__ float4 kv_ld4(const T* p) { return kv_widen(kv_ld_quad(p)); }
+
+// f16: one CTA per SM in the bound (ptxas otherwise caps it at 64 registers and spills at head_dim 128); f32 as it always was
+template <int HD, bool PAGED, typename T>
+__global__ void __launch_bounds__(ATT_NT, std::is_same_v<T, float> ? 0 : 1) attn_decode_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, T* __restrict__ cache_k,
+                                                           T* __restrict__ cache_v, const float* __restrict__ rope, int nh, int nkv,
                                                            int max_ctx, int M, uint8_t* __restrict__ xq, float* __restrict__ attn_out, const PagedKv pg) {
     GlueTrace gt(1);
     pdl_launch_dependents();
@@ -310,11 +337,13 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
         if constexpr (PAGED) return ((size_t)bt[j / pg.block_size] * pg.block_size + (size_t)(j % pg.block_size)) * pstride + (size_t)kvh * HD;
         else return ((size_t)m * max_ctx + (size_t)j) * pstride + (size_t)kvh * HD;
     };
-    float* ck = cache_k;
-    float* cv = cache_v;
+    T* ck = cache_k;
+    T* cv = cache_v;
     const float* rt = rope + (size_t)p * HD;  // [hd/2][2]
 
-    __shared__ __align__(16) float sq[HD], sk[HD], sv[HD];
+    // sk / sv: the new token's k / v as the cache stores them (the f16 cache scores its own row from the rounded values)
+    __shared__ __align__(16) float sq[HD];
+    __shared__ __align__(16) T sk[HD], sv[HD];
     constexpr int NW = ATT_NT / 32;
     __shared__ float s_redf[NW];
     __shared__ double s_redd[NW];
@@ -327,20 +356,22 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
     constexpr int EG = HD / 4;          // output pass: element groups of 4
     constexpr int JG = ATT_NT / EG;     // output pass: position groups (16 for hd 128, 32 for hd 64)
     constexpr int VPF = 8;              // prefetched output-pass iterations (positions < VPF * JG)
+    constexpr int KL = KV_LINE<T>;      // score pass: elements per 16-byte load
     const int part = t & 3;
     const int eg = t % EG, jg = t / EG;
-    float4 kpre[QE / 4], vpre[VPF];
+    kv_line_t<T> kpre[QE / KL];
+    kv_quad_t<T> vpre[VPF];
     float rc = 0.0f, rs = 0.0f;
     {
         const int j = t >> 2;
         if (j < p) {
 #pragma unroll
-            for (int e = 0; e < QE / 4; e++) kpre[e] = *reinterpret_cast<const float4*>(ck + row_of(j) + part * QE + 4 * e);
+            for (int e = 0; e < QE / KL; e++) kpre[e] = kv_ld_line(ck + row_of(j) + part * QE + KL * e);
         }
 #pragma unroll
         for (int it = 0; it < VPF; it++) {
             const int jv = jg + it * JG;
-            if (jv < p) vpre[it] = *reinterpret_cast<const float4*>(cv + row_of(jv) + 4 * eg);
+            if (jv < p) vpre[it] = kv_ld_quad(cv + row_of(jv) + 4 * eg);
         }
         if (t < HD / 2) { rc = rt[2 * t]; rs = rt[2 * t + 1]; }
     }
@@ -356,16 +387,16 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
         sq[2 * t] = __fsub_rn(__fmul_rn(q0, c), __fmul_rn(q1, sn));
         sq[2 * t + 1] = __fadd_rn(__fmul_rn(q0, sn), __fmul_rn(q1, c));
         const float k0 = ksrc[2 * t], k1 = ksrc[2 * t + 1];
-        const float r0 = __fsub_rn(__fmul_rn(k0, c), __fmul_rn(k1, sn)), r1 = __fadd_rn(__fmul_rn(k0, sn), __fmul_rn(k1, c));
+        const T r0 = kv_store_val<T>(__fsub_rn(__fmul_rn(k0, c), __fmul_rn(k1, sn))), r1 = kv_store_val<T>(__fadd_rn(__fmul_rn(k0, sn), __fmul_rn(k1, c)));
         sk[2 * t] = r0; sk[2 * t + 1] = r1;
-        sv[2 * t] = vsrc[2 * t]; sv[2 * t + 1] = vsrc[2 * t + 1];
+        sv[2 * t] = kv_store_val<T>(vsrc[2 * t]); sv[2 * t + 1] = kv_store_val<T>(vsrc[2 * t + 1]);
         if (head % (nh / nkv) == 0) {  // one head of each kv group appends the new k, v
             size_t wrow = row_of(p);
             if constexpr (PAGED) {
                 if (pg.slot_mapping) wrow = (size_t)pg.slot_mapping[m] * pstride + (size_t)kvh * HD;   // the scheduler's slot (batch_decode.rs:84-90)
             }
             ck[wrow + 2 * t] = r0; ck[wrow + 2 * t + 1] = r1;
-            cv[wrow + 2 * t] = vsrc[2 * t]; cv[wrow + 2 * t + 1] = vsrc[2 * t + 1];
+            cv[wrow + 2 * t] = kv_store_val<T>(vsrc[2 * t]); cv[wrow + 2 * t + 1] = kv_store_val<T>(vsrc[2 * t + 1]);
         }
     }
     __syncthreads();
@@ -377,13 +408,26 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
             const int j = j0 + (t >> 2);
             double d0 = 0.0, d1 = 0.0, d2 = 0.0, d3 = 0.0;
             if (j <= p) {
-                const float* kr = (j < p) ? ck + row_of(j) + part * QE : sk + part * QE;  // the new key comes from smem
+                const T* kr = (j < p) ? ck + row_of(j) + part * QE : sk + part * QE;  // the new key comes from smem
                 const float* qq = sq + part * QE;
+                if constexpr (std::is_same_v<T, float>) {
 #pragma unroll
-                for (int e = 0; e < QE; e += 4) {
-                    const float4 kk = (j0 == 0 && j < p) ? kpre[e / 4] : *reinterpret_cast<const float4*>(kr + e);
-                    d0 = fma((double)qq[e + 0], (double)kk.x, d0); d1 = fma((double)qq[e + 1], (double)kk.y, d1);
-                    d2 = fma((double)qq[e + 2], (double)kk.z, d2); d3 = fma((double)qq[e + 3], (double)kk.w, d3);
+                    for (int e = 0; e < QE; e += 4) {
+                        const float4 kk = (j0 == 0 && j < p) ? kpre[e / 4] : *reinterpret_cast<const float4*>(kr + e);
+                        d0 = fma((double)qq[e + 0], (double)kk.x, d0); d1 = fma((double)qq[e + 1], (double)kk.y, d1);
+                        d2 = fma((double)qq[e + 2], (double)kk.z, d2); d3 = fma((double)qq[e + 3], (double)kk.w, d3);
+                    }
+                } else {   // 8 halves per 16-byte load, the same 4 fma chains over e mod 4
+#pragma unroll
+                    for (int e = 0; e < QE; e += KL) {
+                        float kk[KL];
+                        kv_widen((j0 == 0 && j < p) ? kpre[e / KL] : kv_ld_line(kr + e), kk);
+#pragma unroll
+                        for (int i = 0; i < KL; i += 4) {
+                            d0 = fma((double)qq[e + i + 0], (double)kk[i + 0], d0); d1 = fma((double)qq[e + i + 1], (double)kk[i + 1], d1);
+                            d2 = fma((double)qq[e + i + 2], (double)kk[i + 2], d2); d3 = fma((double)qq[e + i + 3], (double)kk[i + 3], d3);
+                        }
+                    }
                 }
             }
             double d = (d0 + d1) + (d2 + d3);
@@ -426,14 +470,14 @@ __global__ void __launch_bounds__(ATT_NT) attn_decode_kernel(const float* __rest
             const int j = jg + it * JG;
             if (j <= p) {
                 const float pj = s_sc[j];
-                const float4 vv = (j < p) ? vpre[it] : *reinterpret_cast<const float4*>(sv + 4 * eg);
+                const float4 vv = (j < p) ? kv_widen(vpre[it]) : kv_ld4(sv + 4 * eg);
                 o0 = fma((double)pj, (double)vv.x, o0); o1 = fma((double)pj, (double)vv.y, o1);
                 o2 = fma((double)pj, (double)vv.z, o2); o3 = fma((double)pj, (double)vv.w, o3);
             }
         }
         for (int j = jg + VPF * JG; j <= p; j += JG) {
             const float pj = s_sc[j];
-            const float4 vv = (j < p) ? *reinterpret_cast<const float4*>(cv + row_of(j) + 4 * eg) : *reinterpret_cast<const float4*>(sv + 4 * eg);
+            const float4 vv = (j < p) ? kv_ld4(cv + row_of(j) + 4 * eg) : kv_ld4(sv + 4 * eg);
             o0 = fma((double)pj, (double)vv.x, o0); o1 = fma((double)pj, (double)vv.y, o1);
             o2 = fma((double)pj, (double)vv.z, o2); o3 = fma((double)pj, (double)vv.w, o3);
         }
@@ -523,9 +567,9 @@ __device__ __forceinline__ int attn_checked_pos(const int* pos, int m, int max_c
     return bad_pos ? 0 : p_raw;
 }
 
-template <int HD, bool PAGED>
-__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, float* __restrict__ cache_k,
-                                                                       float* __restrict__ cache_v, const float* __restrict__ rope, int nh, int nkv, int max_ctx,
+template <int HD, bool PAGED, typename T>
+__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, T* __restrict__ cache_k,
+                                                                       T* __restrict__ cache_v, const float* __restrict__ rope, int nh, int nkv, int max_ctx,
                                                                        const PagedKv pg, const AttnSplitWs ws) {
     pdl_launch_dependents();
     const int kvh = blockIdx.x, m = blockIdx.y, s = blockIdx.z, t = threadIdx.x, warp = t >> 5, lane = t & 31;
@@ -547,8 +591,9 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const f
         else return ((size_t)m * max_ctx + (size_t)j) * pstride + (size_t)kvh * HD;
     };
     const float* rt = rope + (size_t)p * HD;
+    constexpr int KL = KV_LINE<T>;      // elements per 16-byte load
     __shared__ __align__(16) double sq[ATT_SPLIT_GC][4][QP];
-    __shared__ __align__(16) float sk[HD];
+    __shared__ __align__(16) T sk[HD];  // the new key as the cache stores it
     __shared__ float s_red[NW][ATT_SPLIT_GC];
     pdl_wait();
     if (bad_pos) {
@@ -560,7 +605,7 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const f
     if (t < HD / 2) {   // the new key, rotated exactly as attn_decode_kernel does (it is scored from here, never from the cache)
         const float c = rt[2 * t], sn = rt[2 * t + 1];
         const float k0 = ksrc[2 * t], k1 = ksrc[2 * t + 1];
-        const float r0 = __fsub_rn(__fmul_rn(k0, c), __fmul_rn(k1, sn)), r1 = __fadd_rn(__fmul_rn(k0, sn), __fmul_rn(k1, c));
+        const T r0 = kv_store_val<T>(__fsub_rn(__fmul_rn(k0, c), __fmul_rn(k1, sn))), r1 = kv_store_val<T>(__fadd_rn(__fmul_rn(k0, sn), __fmul_rn(k1, c)));
         sk[2 * t] = r0; sk[2 * t + 1] = r1;
         if (owns_p) {
             size_t wrow = row_of(p);
@@ -568,7 +613,7 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const f
                 if (pg.slot_mapping) wrow = (size_t)pg.slot_mapping[m] * pstride + (size_t)kvh * HD;
             }
             cache_k[wrow + 2 * t] = r0; cache_k[wrow + 2 * t + 1] = r1;
-            cache_v[wrow + 2 * t] = vsrc[2 * t]; cache_v[wrow + 2 * t + 1] = vsrc[2 * t + 1];
+            cache_v[wrow + 2 * t] = kv_store_val<T>(vsrc[2 * t]); cache_v[wrow + 2 * t + 1] = kv_store_val<T>(vsrc[2 * t + 1]);
         }
     }
     const float scale = __fdiv_rn(1.0f, __fsqrt_rn((float)HD));
@@ -595,11 +640,21 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const f
             const bool live = j < j1;
             double kd[QE];
             if (live) {
-                const float* kr = (j < p) ? cache_k + row_of(j) + part * QE : sk + part * QE;
+                const T* kr = (j < p) ? cache_k + row_of(j) + part * QE : sk + part * QE;
+                if constexpr (std::is_same_v<T, float>) {
 #pragma unroll
-                for (int e = 0; e < QE; e += 4) {
-                    const float4 kk = *reinterpret_cast<const float4*>(kr + e);
-                    kd[e] = (double)kk.x; kd[e + 1] = (double)kk.y; kd[e + 2] = (double)kk.z; kd[e + 3] = (double)kk.w;
+                    for (int e = 0; e < QE; e += 4) {
+                        const float4 kk = *reinterpret_cast<const float4*>(kr + e);
+                        kd[e] = (double)kk.x; kd[e + 1] = (double)kk.y; kd[e + 2] = (double)kk.z; kd[e + 3] = (double)kk.w;
+                    }
+                } else {   // 8 halves per 16-byte load
+#pragma unroll
+                    for (int e = 0; e < QE; e += KL) {
+                        float kk[KL];
+                        kv_widen(kv_ld_line(kr + e), kk);
+#pragma unroll
+                        for (int i = 0; i < KL; i++) kd[e + i] = (double)kk[i];
+                    }
                 }
             } else {
 #pragma unroll
@@ -643,8 +698,8 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_scores_kernel(const f
     }
 }
 
-template <int HD, bool PAGED>
-__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_pv_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, const float* __restrict__ cache_v,
+template <int HD, bool PAGED, typename T>
+__global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_pv_kernel(const float* __restrict__ qkv, const int* __restrict__ pos, const T* __restrict__ cache_v,
                                                                    int nh, int nkv, int max_ctx, const PagedKv pg, const AttnSplitWs ws) {
     pdl_launch_dependents();
     const int kvh = blockIdx.x, m = blockIdx.y, s = blockIdx.z, t = threadIdx.x, warp = t >> 5, lane = t & 31;
@@ -667,11 +722,11 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_pv_kernel(const float
     };
     __shared__ float sp[ATT_SPLIT_GC][ATT_SPLIT_TILE];
     __shared__ float gmax[ATT_SPLIT_GC];
-    __shared__ __align__(16) float sv[HD];
+    __shared__ __align__(16) T sv[HD];   // the new value as the cache stores it
     __shared__ double s_red[2][NW];
     pdl_wait();
     if (bad_pos || s >= s_eff) return;
-    for (int i = t; i < HD; i += ATT_SPLIT_NT) sv[i] = vsrc[i];
+    for (int i = t; i < HD; i += ATT_SPLIT_NT) sv[i] = kv_store_val<T>(vsrc[i]);
     for (int g0 = 0; g0 < G; g0 += ATT_SPLIT_GC) {
         const int gc = min(ATT_SPLIT_GC, G - g0);
         const size_t hrow = (size_t)m * nh + (size_t)kvh * G + g0;   // first (m, head) row of this pass
@@ -703,7 +758,7 @@ __global__ void __launch_bounds__(ATT_SPLIT_NT) attn_split_pv_kernel(const float
             const int jn = min(ATT_SPLIT_TILE, j1 - jt);
             for (int jj = jg; jj < jn; jj += JG) {
                 const int j = jt + jj;
-                const float4 vv = (j < p) ? *reinterpret_cast<const float4*>(cache_v + row_of(j) + 4 * eg) : *reinterpret_cast<const float4*>(sv + 4 * eg);
+                const float4 vv = (j < p) ? kv_ld4(cache_v + row_of(j) + 4 * eg) : kv_ld4(sv + 4 * eg);
 #pragma unroll
                 for (int g = 0; g < ATT_SPLIT_GC; g++) {
                     const double pj = (double)sp[g][jj];
@@ -801,17 +856,37 @@ static size_t attn_split_layout(int64_t nh, int64_t hd, int64_t max_ctx, int64_t
     return b_sc + b_mx + b_ps + b_pv;
 }
 
-template <int HD, bool PAGED>
-static cudaError_t launch_attn_split(const float* qkv, const int* pos, float* ck, float* cv, const float* rope, int nh, int nkv, int max_ctx, int M,
+template <int HD, bool PAGED, typename T>
+static cudaError_t launch_attn_split(const float* qkv, const int* pos, T* ck, T* cv, const float* rope, int nh, int nkv, int max_ctx, int M,
                                      uint8_t* xq, float* attn_out, const PagedKv& pg, const AttnSplitWs& ws, cudaStream_t st) {
     const int s_max = attn_split_max(max_ctx);
     const dim3 grid((unsigned)nkv, (unsigned)M, (unsigned)s_max);
-    cudaError_t e = launch_pdl(attn_split_scores_kernel<HD, PAGED>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, ck, cv, rope, nh, nkv, max_ctx, pg, ws);
+    cudaError_t e = launch_pdl(attn_split_scores_kernel<HD, PAGED, T>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, ck, cv, rope, nh, nkv, max_ctx, pg, ws);
     if (e == cudaSuccess)
-        e = launch_pdl(attn_split_pv_kernel<HD, PAGED>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, (const float*)cv, nh, nkv, max_ctx, pg, ws);
+        e = launch_pdl(attn_split_pv_kernel<HD, PAGED, T>, grid, dim3(ATT_SPLIT_NT), 0, st, qkv, pos, (const T*)cv, nh, nkv, max_ctx, pg, ws);
     if (e == cudaSuccess)
         e = launch_pdl(attn_split_combine_kernel<HD, PAGED>, dim3((unsigned)nh, (unsigned)M), dim3(HD), 0, st, pos, nh, max_ctx, s_max, M, pg, ws, xq, attn_out);
     return e;
+}
+
+template <int HD, bool PAGED, typename T>
+static cudaError_t launch_attn_single(const float* qkv, const int* pos, T* ck, T* cv, const float* rope, int nh, int nkv, int max_ctx, int M,
+                                      uint8_t* xq, float* attn_out, const PagedKv& pg, cudaStream_t st) {
+    const size_t smem = (size_t)max_ctx * sizeof(float);
+    if (smem > 48 * 1024) cudaFuncSetAttribute(attn_decode_kernel<HD, PAGED, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    return launch_pdl(attn_decode_kernel<HD, PAGED, T>, dim3((unsigned)nh, (unsigned)M), dim3(ATT_NT), smem, st, qkv, pos, ck, cv, rope, nh, nkv, max_ctx, M,
+                      xq, attn_out, pg);
+}
+
+template <typename T>
+static cudaError_t launch_attn_split_hd(int32_t hd, const float* qkv, const int32_t* pos, T* ck, T* cv, const float* rope, int32_t nh, int32_t nkv,
+                                        int max_ctx, int M, uint8_t* xq, float* attn_out, const PagedKv& pg, const AttnSplitWs& ws, cudaStream_t st) {
+    const bool paged = pg.block_table != nullptr;
+    if (hd == 128)
+        return paged ? launch_attn_split<128, true>(qkv, pos, ck, cv, rope, nh, nkv, max_ctx, M, xq, attn_out, pg, ws, st)
+                     : launch_attn_split<128, false>(qkv, pos, ck, cv, rope, nh, nkv, max_ctx, M, xq, attn_out, pg, ws, st);
+    return paged ? launch_attn_split<64, true>(qkv, pos, ck, cv, rope, nh, nkv, max_ctx, M, xq, attn_out, pg, ws, st)
+                 : launch_attn_split<64, false>(qkv, pos, ck, cv, rope, nh, nkv, max_ctx, M, xq, attn_out, pg, ws, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1014,60 +1089,84 @@ int32_t b200q_swiglu_f32_interleaved(const float* gate_up, int64_t F, int64_t M,
     return e == cudaSuccess ? B200Q_OK : B200Q_ERR_CUDA;
 }
 
+// KV cache element type and alignment: every attention form vector-loads 16 bytes of a cache row (the row starts are 16-byte
+// aligned for head_dim 64 / 128 in both dtypes, so the base pointers must be too)
+static int32_t attn_kv_check(const void* ck, const void* cv, int32_t kv_dtype, const char* who) {
+    if (kv_dtype != B200Q_F32 && kv_dtype != B200Q_F16) return set_error(B200Q_ERR_UNSUPPORTED, "%s: kv_dtype %d (B200Q_F32 or B200Q_F16)", who, (int)kv_dtype);
+    if (((uintptr_t)ck | (uintptr_t)cv) & 15) return set_error(B200Q_ERR_INVALID_ARG, "%s: KV cache pointers must be 16-byte aligned", who);
+    return B200Q_OK;
+}
+
+static int32_t attn_single_dispatch(const float* qkv, const int32_t* pos, void* ck, void* cv, int32_t kv_dtype, const float* rope, int32_t nh, int32_t nkv,
+                                    int32_t hd, int64_t max_ctx, int64_t M, void* xq, float* attn_out, const PagedKv& pg, void* stream, const char* who) {
+    if (max_ctx > ATTN_SINGLE_MAX_CTX) return set_error(B200Q_ERR_UNSUPPORTED, "%s: max_ctx %lld > %d (use the split form)", who, (long long)max_ctx, ATTN_SINGLE_MAX_CTX);
+    if (hd != 64 && hd != 128) return set_error(B200Q_ERR_UNSUPPORTED, "%s: head_dim %d (64 or 128)", who, (int)hd);
+    const int32_t rc = attn_kv_check(ck, cv, kv_dtype, who);
+    if (rc != B200Q_OK) return rc;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const bool paged = pg.block_table != nullptr;
+    const int mc = (int)max_ctx, m = (int)M;
+    uint8_t* x = (uint8_t*)xq;
+    cudaError_t e;
+    if (kv_dtype == B200Q_F16) {
+        __half* k = (__half*)ck;
+        __half* v = (__half*)cv;
+        if (hd == 128)
+            e = paged ? launch_attn_single<128, true>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st)
+                      : launch_attn_single<128, false>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st);
+        else
+            e = paged ? launch_attn_single<64, true>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st)
+                      : launch_attn_single<64, false>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st);
+    } else {
+        float* k = (float*)ck;
+        float* v = (float*)cv;
+        if (hd == 128)
+            e = paged ? launch_attn_single<128, true>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st)
+                      : launch_attn_single<128, false>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st);
+        else
+            e = paged ? launch_attn_single<64, true>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st)
+                      : launch_attn_single<64, false>(qkv, pos, k, v, rope, nh, nkv, mc, m, x, attn_out, pg, st);
+    }
+    return e == cudaSuccess ? B200Q_OK : set_error(B200Q_ERR_CUDA, "%s launch: %s", who, cudaGetErrorString(e));
+}
+
+int32_t b200q_attn_decode_kv(const float* qkv, const int32_t* pos, void* cache_k, void* cache_v, int32_t kv_dtype, const float* rope_table, int32_t n_heads,
+                             int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* stream) {
+    if (!qkv || !pos || !cache_k || !cache_v || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 || max_ctx <= 0)
+        return set_error(B200Q_ERR_INVALID_ARG, "attn_decode: bad arguments");
+    if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode: n_heads * head_dim not a multiple of %d", CHUNK_K);
+    const PagedKv none{nullptr, nullptr, 0, 0};
+    return attn_single_dispatch(qkv, pos, cache_k, cache_v, kv_dtype, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, none, stream,
+                                "attn_decode");
+}
+
 int32_t b200q_attn_decode(const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table, int32_t n_heads,
                           int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* stream) {
-    if (!qkv || !pos || !cache_k || !cache_v || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 || max_ctx <= 0)
-        return B200Q_ERR_INVALID_ARG;
-    if (((int64_t)n_heads * head_dim) % CHUNK_K) return B200Q_ERR_INVALID_ARG;
-    if (max_ctx > ATTN_SINGLE_MAX_CTX) return B200Q_ERR_UNSUPPORTED;
-    cudaError_t e;
-    dim3 grid((unsigned)n_heads, (unsigned)M);
-    size_t smem = (size_t)max_ctx * sizeof(float);
-    const PagedKv none{nullptr, nullptr, 0, 0};
-    if (head_dim == 128) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(attn_decode_kernel<128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        e = launch_pdl(attn_decode_kernel<128, false>, grid, dim3(ATT_NT), smem, (cudaStream_t)stream, qkv, (const int*)pos, cache_k, cache_v, rope_table,
-                       (int)n_heads, (int)n_kv_heads, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, (const PagedKv)none);
-    } else if (head_dim == 64) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(attn_decode_kernel<64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        e = launch_pdl(attn_decode_kernel<64, false>, grid, dim3(ATT_NT), smem, (cudaStream_t)stream, qkv, (const int*)pos, cache_k, cache_v, rope_table,
-                       (int)n_heads, (int)n_kv_heads, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, (const PagedKv)none);
-    } else {
-        return B200Q_ERR_UNSUPPORTED;
-    }
-    return e == cudaSuccess ? B200Q_OK : B200Q_ERR_CUDA;
+    return b200q_attn_decode_kv(qkv, pos, cache_k, cache_v, B200Q_F32, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, stream);
 }
 
 /* Paged form (reference forward_with_paged_kv_cache, src/engine/batch_decode.rs:115-147): k_pool / v_pool are
- * [num_blocks][block_size][nkv][hd] f32 pools shared by all sequences, block_table int32 [M][max_blocks] (padding entries are
+ * [num_blocks][block_size][nkv][hd] pools shared by all sequences, block_table int32 [M][max_blocks] (padding entries are
  * never read: only blocks below pos[m] / block_size are), slot_mapping int32 [M] = block * block_size + offset of the NEW
  * token (nullable: derived from block_table and pos).  pos[m] = sequence length - 1.  A slot of -1 or a position >=
  * max_blocks * block_size writes nothing and raises the sticky device error (b200q_decode_error). */
+int32_t b200q_attn_decode_paged_kv(const float* qkv, const int32_t* pos, void* k_pool, void* v_pool, int32_t kv_dtype, const int32_t* block_table,
+                                   const int32_t* slot_mapping, int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads,
+                                   int32_t n_kv_heads, int32_t head_dim, int64_t M, void* xq, float* attn_out, void* stream) {
+    if (!qkv || !pos || !k_pool || !v_pool || !block_table || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 ||
+        block_size <= 0 || max_blocks <= 0)
+        return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged: bad arguments");
+    if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged: n_heads * head_dim not a multiple of %d", CHUNK_K);
+    const PagedKv pg{block_table, slot_mapping, block_size, max_blocks};
+    return attn_single_dispatch(qkv, pos, k_pool, v_pool, kv_dtype, rope_table, n_heads, n_kv_heads, head_dim, (int64_t)block_size * max_blocks, M, xq,
+                                attn_out, pg, stream, "attn_decode_paged");
+}
+
 int32_t b200q_attn_decode_paged(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
                                 int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
                                 int64_t M, void* xq, float* attn_out, void* stream) {
-    if (!qkv || !pos || !k_pool || !v_pool || !block_table || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 ||
-        block_size <= 0 || max_blocks <= 0)
-        return B200Q_ERR_INVALID_ARG;
-    if (((int64_t)n_heads * head_dim) % CHUNK_K) return B200Q_ERR_INVALID_ARG;
-    const int64_t max_ctx = (int64_t)block_size * max_blocks;
-    if (max_ctx > ATTN_SINGLE_MAX_CTX) return B200Q_ERR_UNSUPPORTED;
-    cudaError_t e;
-    dim3 grid((unsigned)n_heads, (unsigned)M);
-    size_t smem = (size_t)max_ctx * sizeof(float);
-    const PagedKv pg{block_table, slot_mapping, block_size, max_blocks};
-    if (head_dim == 128) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(attn_decode_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        e = launch_pdl(attn_decode_kernel<128, true>, grid, dim3(ATT_NT), smem, (cudaStream_t)stream, qkv, (const int*)pos, k_pool, v_pool, rope_table,
-                       (int)n_heads, (int)n_kv_heads, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, (const PagedKv)pg);
-    } else if (head_dim == 64) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(attn_decode_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        e = launch_pdl(attn_decode_kernel<64, true>, grid, dim3(ATT_NT), smem, (cudaStream_t)stream, qkv, (const int*)pos, k_pool, v_pool, rope_table,
-                       (int)n_heads, (int)n_kv_heads, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, (const PagedKv)pg);
-    } else {
-        return B200Q_ERR_UNSUPPORTED;
-    }
-    return e == cudaSuccess ? B200Q_OK : B200Q_ERR_CUDA;
+    return b200q_attn_decode_paged_kv(qkv, pos, k_pool, v_pool, B200Q_F32, block_table, slot_mapping, block_size, max_blocks, rope_table, n_heads, n_kv_heads,
+                                      head_dim, M, xq, attn_out, stream);
 }
 
 int32_t b200q_attn_decode_max_ctx(void) { return ATTN_SINGLE_MAX_CTX; }
@@ -1077,50 +1176,63 @@ size_t b200q_attn_split_workspace_bytes(int32_t n_heads, int32_t n_kv_heads, int
     return attn_split_layout(n_heads, head_dim, max_ctx, M, nullptr, nullptr);
 }
 
-static int32_t attn_split_dispatch(const float* qkv, const int32_t* pos, float* ck, float* cv, const float* rope, int32_t nh, int32_t nkv, int32_t hd,
-                                   int64_t max_ctx, int64_t M, void* xq, float* attn_out, const PagedKv& pg, void* workspace, size_t workspace_bytes,
-                                   void* stream, const char* who) {
+static int32_t attn_split_dispatch(const float* qkv, const int32_t* pos, void* ck, void* cv, int32_t kv_dtype, const float* rope, int32_t nh, int32_t nkv,
+                                   int32_t hd, int64_t max_ctx, int64_t M, void* xq, float* attn_out, const PagedKv& pg, void* workspace,
+                                   size_t workspace_bytes, void* stream, const char* who) {
     if (hd != 64 && hd != 128) return set_error(B200Q_ERR_UNSUPPORTED, "%s: head_dim %d (64 or 128)", who, (int)hd);
     if (max_ctx > INT32_MAX || M > 65535) return set_error(B200Q_ERR_INVALID_ARG, "%s: max_ctx %lld / M %lld out of range", who, (long long)max_ctx, (long long)M);
+    const int32_t rc = attn_kv_check(ck, cv, kv_dtype, who);
+    if (rc != B200Q_OK) return rc;
     AttnSplitWs ws;
     const size_t need = attn_split_layout(nh, hd, max_ctx, M, (uint8_t*)workspace, &ws);
     if (!workspace || workspace_bytes < need)
         return set_error(B200Q_ERR_WORKSPACE, "%s: workspace of %zu bytes, %zu needed (b200q_attn_split_workspace_bytes)", who, workspace_bytes, need);
-    cudaError_t e;
     const cudaStream_t st = (cudaStream_t)stream;
-    const bool paged = pg.block_table != nullptr;
-    if (hd == 128)
-        e = paged ? launch_attn_split<128, true>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st)
-                  : launch_attn_split<128, false>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st);
-    else
-        e = paged ? launch_attn_split<64, true>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st)
-                  : launch_attn_split<64, false>(qkv, pos, ck, cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st);
+    const cudaError_t e =
+        kv_dtype == B200Q_F16
+            ? launch_attn_split_hd(hd, qkv, pos, (__half*)ck, (__half*)cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st)
+            : launch_attn_split_hd(hd, qkv, pos, (float*)ck, (float*)cv, rope, nh, nkv, (int)max_ctx, (int)M, (uint8_t*)xq, attn_out, pg, ws, st);
     return e == cudaSuccess ? B200Q_OK : set_error(B200Q_ERR_CUDA, "%s launch: %s", who, cudaGetErrorString(e));
 }
 
-/* Split-context form of b200q_attn_decode for any max_ctx >= 1 (same arguments, same results up to the order of the f64 sums). */
-int32_t b200q_attn_decode_split(const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table, int32_t n_heads,
-                                int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* workspace,
-                                size_t workspace_bytes, void* stream) {
+/* Split-context form of b200q_attn_decode_kv for any max_ctx >= 1 (same arguments, same results up to the order of the f64 sums). */
+int32_t b200q_attn_decode_split_kv(const float* qkv, const int32_t* pos, void* cache_k, void* cache_v, int32_t kv_dtype, const float* rope_table,
+                                   int32_t n_heads, int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out,
+                                   void* workspace, size_t workspace_bytes, void* stream) {
     if (!qkv || !pos || !cache_k || !cache_v || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 || max_ctx <= 0)
         return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_split: bad arguments");
     if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_split: n_heads * head_dim not a multiple of %d", CHUNK_K);
     const PagedKv none{nullptr, nullptr, 0, 0};
-    return attn_split_dispatch(qkv, pos, cache_k, cache_v, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, none, workspace,
+    return attn_split_dispatch(qkv, pos, cache_k, cache_v, kv_dtype, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, none, workspace,
                                workspace_bytes, stream, "attn_decode_split");
 }
 
-/* Split-context form of b200q_attn_decode_paged; max_ctx = block_size * max_blocks sizes the workspace. */
-int32_t b200q_attn_decode_paged_split(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
-                                      int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
-                                      int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes, void* stream) {
+int32_t b200q_attn_decode_split(const float* qkv, const int32_t* pos, float* cache_k, float* cache_v, const float* rope_table, int32_t n_heads,
+                                int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+    return b200q_attn_decode_split_kv(qkv, pos, cache_k, cache_v, B200Q_F32, rope_table, n_heads, n_kv_heads, head_dim, max_ctx, M, xq, attn_out, workspace,
+                                      workspace_bytes, stream);
+}
+
+/* Split-context form of b200q_attn_decode_paged_kv; max_ctx = block_size * max_blocks sizes the workspace. */
+int32_t b200q_attn_decode_paged_split_kv(const float* qkv, const int32_t* pos, void* k_pool, void* v_pool, int32_t kv_dtype, const int32_t* block_table,
+                                         const int32_t* slot_mapping, int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads,
+                                         int32_t n_kv_heads, int32_t head_dim, int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
     if (!qkv || !pos || !k_pool || !v_pool || !block_table || !rope_table || (!xq && !attn_out) || n_heads <= 0 || n_kv_heads <= 0 || n_heads % n_kv_heads || M <= 0 ||
         block_size <= 0 || max_blocks <= 0)
         return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged_split: bad arguments");
     if (((int64_t)n_heads * head_dim) % CHUNK_K) return set_error(B200Q_ERR_INVALID_ARG, "attn_decode_paged_split: n_heads * head_dim not a multiple of %d", CHUNK_K);
     const PagedKv pg{block_table, slot_mapping, block_size, max_blocks};
-    return attn_split_dispatch(qkv, pos, k_pool, v_pool, rope_table, n_heads, n_kv_heads, head_dim, (int64_t)block_size * max_blocks, M, xq, attn_out, pg,
-                               workspace, workspace_bytes, stream, "attn_decode_paged_split");
+    return attn_split_dispatch(qkv, pos, k_pool, v_pool, kv_dtype, rope_table, n_heads, n_kv_heads, head_dim, (int64_t)block_size * max_blocks, M, xq, attn_out,
+                               pg, workspace, workspace_bytes, stream, "attn_decode_paged_split");
+}
+
+int32_t b200q_attn_decode_paged_split(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
+                                      int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
+                                      int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes, void* stream) {
+    return b200q_attn_decode_paged_split_kv(qkv, pos, k_pool, v_pool, B200Q_F32, block_table, slot_mapping, block_size, max_blocks, rope_table, n_heads,
+                                            n_kv_heads, head_dim, M, xq, attn_out, workspace, workspace_bytes, stream);
 }
 
 /* Reads and clears the sticky device error word of the CURRENT device (synchronises the device: call it outside

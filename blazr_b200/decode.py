@@ -55,6 +55,16 @@ PRESETS: Dict[str, ModelConfig] = {
 }
 
 
+# Decoder(kv_dtype=...): torch element type of the KV cache and the b200q_dtype the *_kv attention entry points take
+KV_DTYPES = {"f32": (torch.float32, 0), "f16": (torch.float16, 1)}
+
+
+def kv_round(x: torch.Tensor) -> torch.Tensor:
+    """The f16 KV cache element rule of the attention kernels: f16_rn(clamp(x, +-65504)), NaN -> -65504 (torch's conversion
+    rounds to nearest even, as __float2half_rn does)"""
+    return x.nan_to_num(nan=-65504.0).clamp(-65504.0, 65504.0).to(torch.float16)
+
+
 def rope_table(max_ctx: int, head_dim: int, theta: float, factors=None) -> np.ndarray:
     """[max_ctx, hd/2, 2] f32 (cos, sin) of pos * theta^(-2i/hd) / factors[i], computed in f64 and rounded once.  The same
     formula is restated in oracle/model.py (unscaled) and tests/rope_ref.py (with factors); a table (instead of device
@@ -193,15 +203,21 @@ class Decoder:
 
     def __init__(self, client: ops.B200Client, cfg: ModelConfig, scheme: str, batch: int = 1, max_ctx: int = 512,
                  host: Optional[HostModel] = None, seed: int = 0xB200, tp_rank: int = 0, tp_world: int = 1, group=None,
-                 paged: bool = False, block_size: int = 16, emulate_shard: bool = False):
+                 paged: bool = False, block_size: int = 16, emulate_shard: bool = False, kv_dtype: str = "f32"):
         """paged: KV cache as block pools + block table (reference InferenceConfig.paged_attention / block_size = 16,
         src/config/inference.rs:94-98; forward_with_paged_kv_cache, src/engine/batch_decode.rs:137-147) instead of one
         contiguous [max_ctx] region per sequence.  emulate_shard: build rank tp_rank's shard of a tp_world-way tensor-parallel
         model but run it ALONE on this GPU through the same fused-exchange kernels (world-1 communicator): the per-rank
         latency structure of TP-N measured on one GPU (tools / profiling only; the logits are those of the shard).
         The block table is pre-populated with a shuffled assignment of the pool's
-        blocks; a scheduler may overwrite `block_table` / `slot_mapping` between steps (blazr_b200/batch.py builds them)."""
+        blocks; a scheduler may overwrite `block_table` / `slot_mapping` between steps (blazr_b200/batch.py builds them).
+        kv_dtype: "f32" (default) or "f16" KV cache; f16 halves the cache and stores f16_rn(clamp(x, +-65504)) of every K / V
+        element (include/b200q.h, b200q_attn_decode_kv)."""
         assert 1 <= batch <= 256
+        if kv_dtype not in KV_DTYPES:
+            raise ValueError(f"kv_dtype {kv_dtype!r}: one of {sorted(KV_DTYPES)}")
+        self.kv_dtype = kv_dtype
+        kv_t = KV_DTYPES[kv_dtype][0]
         # M <= 4: dp4a matvec on int8 activation records (bit-exact contract); M > 4 (batched decode, reference
         # src/engine/batch_decode.rs:115-147): tcgen05 dequant-GEMM on f32 activations (1e-2 tolerance contract)
         self.wide = batch > 4
@@ -258,12 +274,13 @@ class Decoder:
             lay["mlp_norm"] = torch.from_numpy(mn).to(dev)
             if paged:  # block pools [num_blocks][block_size][nkv][hd]
                 nblk = M * (-(-max_ctx // block_size))
-                lay["ck"] = torch.zeros((nblk, block_size, self.nkv, hd), dtype=torch.float32, device=dev)
-                lay["cv"] = torch.zeros((nblk, block_size, self.nkv, hd), dtype=torch.float32, device=dev)
+                lay["ck"] = torch.zeros((nblk, block_size, self.nkv, hd), dtype=kv_t, device=dev)
+                lay["cv"] = torch.zeros((nblk, block_size, self.nkv, hd), dtype=kv_t, device=dev)
             else:
-                lay["ck"] = torch.zeros((M, max_ctx, self.nkv, hd), dtype=torch.float32, device=dev)
-                lay["cv"] = torch.zeros((M, max_ctx, self.nkv, hd), dtype=torch.float32, device=dev)
+                lay["ck"] = torch.zeros((M, max_ctx, self.nkv, hd), dtype=kv_t, device=dev)
+                lay["cv"] = torch.zeros((M, max_ctx, self.nkv, hd), dtype=kv_t, device=dev)
             self.layers.append(lay)
+        self.kv_cache_bytes = sum(lay[c].numel() * lay[c].element_size() for lay in self.layers for c in ("ck", "cv"))
         self.final_norm = torch.from_numpy(host.final_norm if host else np.ones(H, np.float32)).to(dev)
         self.rope = torch.from_numpy(rope_table(max_ctx, hd, cfg.rope_theta, cfg.rope_freq_factors)).to(dev)
         # decode attention: the single-CTA kernel holds every score of a (head, sequence) in shared memory; past its limit the
@@ -460,29 +477,30 @@ class Decoder:
         L, cfg, M = ops.lib(), self.cfg, self.M
         P = lambda t: C.c_void_p(t.data_ptr())
         xq, ao = (None, P(self.xq_attn)) if self.wide else (P(self.xq_attn), None)
+        kvt = C.c_int32(KV_DTYPES[self.kv_dtype][1])
         if self.attn_split:
             ws, wsb = P(self.attn_ws), C.c_size_t(self.attn_ws.numel())
             if self.paged:
-                ops._check(L.b200q_attn_decode_paged_split(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.block_table),
-                                                           P(self.slot_mapping) if self.slot_mapping is not None else None,
-                                                           C.c_int32(self.block_size), C.c_int32(self.max_blocks), P(self.rope), C.c_int32(self.nh),
-                                                           C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int64(M), xq, ao, ws, wsb, st))
+                ops._check(L.b200q_attn_decode_paged_split_kv(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), kvt, P(self.block_table),
+                                                              P(self.slot_mapping) if self.slot_mapping is not None else None,
+                                                              C.c_int32(self.block_size), C.c_int32(self.max_blocks), P(self.rope), C.c_int32(self.nh),
+                                                              C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int64(M), xq, ao, ws, wsb, st))
             else:
-                ops._check(L.b200q_attn_decode_split(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.rope), C.c_int32(self.nh),
-                                                     C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M), xq, ao,
-                                                     ws, wsb, st))
+                ops._check(L.b200q_attn_decode_split_kv(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), kvt, P(self.rope), C.c_int32(self.nh),
+                                                        C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M), xq, ao,
+                                                        ws, wsb, st))
             return
         if self.paged:
-            ops._check(L.b200q_attn_decode_paged(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.block_table),
-                                                 P(self.slot_mapping) if self.slot_mapping is not None else None, C.c_int32(self.block_size),
-                                                 C.c_int32(self.max_blocks), P(self.rope), C.c_int32(self.nh), C.c_int32(self.nkv),
-                                                 C.c_int32(cfg.head_dim), C.c_int64(M), xq, ao, st))
+            ops._check(L.b200q_attn_decode_paged_kv(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), kvt, P(self.block_table),
+                                                    P(self.slot_mapping) if self.slot_mapping is not None else None, C.c_int32(self.block_size),
+                                                    C.c_int32(self.max_blocks), P(self.rope), C.c_int32(self.nh), C.c_int32(self.nkv),
+                                                    C.c_int32(cfg.head_dim), C.c_int64(M), xq, ao, st))
         else:
-            ops._check(L.b200q_attn_decode(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), P(self.rope), C.c_int32(self.nh),
-                                           C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M), xq, ao, st))
+            ops._check(L.b200q_attn_decode_kv(P(self.qkv), P(self.pos), P(lay["ck"]), P(lay["cv"]), kvt, P(self.rope), C.c_int32(self.nh),
+                                              C.c_int32(self.nkv), C.c_int32(cfg.head_dim), C.c_int32(self.max_ctx), C.c_int64(M), xq, ao, st))
 
     def kv_rows(self, lay, seq: int, S: int):
-        """(K, V) rows [S, nkv, hd] of positions 0..S-1 of sequence `seq`, whatever the cache layout"""
+        """(K, V) rows [S, nkv, hd] of positions 0..S-1 of sequence `seq`, whatever the cache layout, in the stored dtype"""
         if not self.paged:
             return lay["ck"][seq, :S], lay["cv"][seq, :S]
         j = torch.arange(S, device=self.dev)
@@ -491,8 +509,10 @@ class Decoder:
         return lay["ck"].view(-1, nkv, hd)[idx], lay["cv"].view(-1, nkv, hd)[idx]
 
     def _kv_write(self, lay, seq: int, k: torch.Tensor, v: torch.Tensor):
-        """prefill: store K (rotated) / V rows [S, nkv, hd] of sequence `seq`"""
+        """prefill: store K (rotated) / V rows [S, nkv, hd] of sequence `seq` (f32 values; an f16 cache stores kv_round of them)"""
         S = k.shape[0]
+        if self.kv_dtype == "f16":
+            k, v = kv_round(k), kv_round(v)
         if not self.paged:
             lay["ck"][seq, :S].copy_(k)
             lay["cv"][seq, :S].copy_(v)

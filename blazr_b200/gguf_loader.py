@@ -368,15 +368,16 @@ def host_model_from_gguf(g: Gguf, client=None):
     return hm
 
 
-def load_gguf(client, path: str, batch: int = 1, max_ctx: int = 512, tp_rank: int = 0, tp_world: int = 1, group=None):
+def load_gguf(client, path: str, batch: int = 1, max_ctx: int = 512, tp_rank: int = 0, tp_world: int = 1, group=None, kv_dtype: str = "f32"):
     """reference gguf.rs:20-44: open, derive the config from the metadata, upload every tensor, build the model.
-    Returns (Decoder, ModelConfig).  Each TP rank uploads only its shard of the mmapped blocks (the reference makes
+    Returns (Decoder, ModelConfig); kv_dtype "f16" halves the KV cache (Decoder).  Each TP rank uploads only its shard of the mmapped blocks (the reference makes
     every rank read the whole file, regular.rs:152)."""
     from .decode import Decoder
 
     g = Gguf.open(path)
     hm = host_model_from_gguf(g, client)
-    dec = Decoder(client, hm.cfg, hm.scheme, batch=batch, max_ctx=max_ctx, host=hm, tp_rank=tp_rank, tp_world=tp_world, group=group)
+    dec = Decoder(client, hm.cfg, hm.scheme, batch=batch, max_ctx=max_ctx, host=hm, tp_rank=tp_rank, tp_world=tp_world, group=group,
+                  kv_dtype=kv_dtype)
     return dec, hm.cfg
 
 

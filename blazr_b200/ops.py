@@ -55,6 +55,7 @@ EXPORTS = [
     "b200q_act_bytes", "b200q_quantize_act", "b200q_matmul_q8", "b200q_matmul_path", "b200q_dequantize", "b200q_act_unpack",
     "b200q_int_partials", "b200q_launch_count", "b200q_add_rmsnorm_quant", "b200q_swiglu_quant", "b200q_attn_decode", "b200q_attn_decode_paged",
     "b200q_attn_decode_max_ctx", "b200q_attn_split_workspace_bytes", "b200q_attn_decode_split", "b200q_attn_decode_paged_split",
+    "b200q_attn_decode_kv", "b200q_attn_decode_paged_kv", "b200q_attn_decode_split_kv", "b200q_attn_decode_paged_split_kv",
     "b200q_argmax", "b200q_decode_error", "b200q_embed", "b200q_matmul_norm", "b200q_matmul_swiglu",
     "b200q_swiglu_f32", "b200q_swiglu_f32_interleaved", "b200q_gate_up_row", "b200q_matmul_q8_swiglu", "b200q_matmul_norm_swiglu", "b200q_moe_matmul_q8_swiglu",
     "b200q_comm_create", "b200q_comm_handle", "b200q_comm_connect", "b200q_allreduce_f64", "b200q_comm_free", "b200q_comm_gather_ptr",

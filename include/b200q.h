@@ -297,6 +297,26 @@ int32_t b200q_attn_decode_split(const float* qkv, const int32_t* pos, float* cac
 int32_t b200q_attn_decode_paged_split(const float* qkv, const int32_t* pos, float* k_pool, float* v_pool, const int32_t* block_table, const int32_t* slot_mapping,
                                       int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads, int32_t n_kv_heads, int32_t head_dim,
                                       int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The four attention forms above with the KV cache in a chosen element type: cache_k / cache_v (k_pool / v_pool) are arrays
+ * of kv_dtype elements in the same layouts, followed by the same arguments.  kv_dtype B200Q_F32 is exactly the f32-named
+ * function (they are its B200Q_F32 case); B200Q_F16 halves the cache.  An f16 element is stored as
+ * f16_rn(clamp(x, -65504, 65504)) of the f32 value the f32 form would store (the rotated k, the raw v; NaN stores -65504), and
+ * the step that appends row p scores and weights its own k / v from those rounded values, so a row reads the same at every
+ * step.  Every loaded element widens exactly to f32; all arithmetic after the load is that of the f32 forms.  Another kv_dtype
+ * -> B200Q_ERR_UNSUPPORTED; cache pointers not 16-byte aligned -> B200Q_ERR_INVALID_ARG (both before any launch).  The split
+ * workspace does not depend on kv_dtype. */
+int32_t b200q_attn_decode_kv(const float* qkv, const int32_t* pos, void* cache_k, void* cache_v, int32_t kv_dtype, const float* rope_table, int32_t n_heads,
+                             int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out, void* stream);
+int32_t b200q_attn_decode_paged_kv(const float* qkv, const int32_t* pos, void* k_pool, void* v_pool, int32_t kv_dtype, const int32_t* block_table,
+                                   const int32_t* slot_mapping, int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads,
+                                   int32_t n_kv_heads, int32_t head_dim, int64_t M, void* xq, float* attn_out, void* stream);
+int32_t b200q_attn_decode_split_kv(const float* qkv, const int32_t* pos, void* cache_k, void* cache_v, int32_t kv_dtype, const float* rope_table,
+                                   int32_t n_heads, int32_t n_kv_heads, int32_t head_dim, int32_t max_ctx, int64_t M, void* xq, float* attn_out,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+int32_t b200q_attn_decode_paged_split_kv(const float* qkv, const int32_t* pos, void* k_pool, void* v_pool, int32_t kv_dtype, const int32_t* block_table,
+                                         const int32_t* slot_mapping, int32_t block_size, int32_t max_blocks, const float* rope_table, int32_t n_heads,
+                                         int32_t n_kv_heads, int32_t head_dim, int64_t M, void* xq, float* attn_out, void* workspace, size_t workspace_bytes,
+                                         void* stream);
 /* A position pos[m] outside [0, max_ctx) makes b200q_attn_decode write nothing and raise a sticky per-device error
  * word instead of indexing past the KV cache.  b200q_decode_error reads and clears it for the current device
  * (synchronises the device: not capturable; call it after a generate loop).  bit 0 = position out of range. */
